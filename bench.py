@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            our CUDA path (one process per GPU under torchrun)
     python bench.py --impl reference --steps K --warmup W    the CPU arm: the oracle port on the host cores
     python bench.py --config {1,2,3,4} ...                   which BASELINE.json configs[] entry (default 1)
+    python bench.py ... --dump-outputs DIR                   also write the last timed step's outputs as DIR/<name>.npy
 
 configs[1] (default, the headline): a step is one pass of the hot path (sample K hypotheses -> collapse -> edit
 distance -> reward -> baseline -> REINFORCE gradient, plus CTC alpha-beta loss and gradient; loss scalar + dlogits
@@ -57,7 +58,13 @@ def parse():
     ap.add_argument("--w-pg", type=float, default=None, help="diagnosis: override the PG weight (0 drops the PG role)")
     ap.add_argument("--w-ctc", type=float, default=None, help="diagnosis: override the CTC weight (0 drops the CTC role)")
     ap.add_argument("--python-loop", action="store_true", help="one functional.pg_ctc_step call per step (round-1 loop)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy; configs[1] and [2]")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "ours" or args.config not in (1, 2)):
+        ap.error("--dump-outputs covers the GPU path of configs[1] and configs[2]")
     sh = SHAPES.get(args.config, SHAPES[1])
     for k in ("batch", "T", "V", "K", "L"):
         if not getattr(args, k):
@@ -118,6 +125,27 @@ def traffic_from_profile(workload_key):
 def pool_size(args):
     bytes_logits = args.batch * args.T * args.V * 4
     return max(2, -(-int(1.25 * L2_BYTES) // bytes_logits)), bytes_logits      # rotating inputs: pool footprint > L2
+
+
+DUMP_BYTES = 64 * 2**20
+
+
+def dump_outputs(directory, outputs):
+    """outputs: name -> torch tensor, as the step returned them.  Written as float32 (float64 stays float64, integers
+    become float64, which holds them exactly).  Past DUMP_BYTES in all, an array over its share of the budget is
+    replaced by the same seeded sample of its flattened elements on every run, so that two builds stay comparable."""
+    arrays = {}
+    for name, t in outputs.items():
+        a = t.detach().cpu().numpy()
+        arrays[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(directory, exist_ok=True)
+    for name, a in sorted(arrays.items()):
+        share = DUMP_BYTES // len(arrays) // a.itemsize
+        if total > DUMP_BYTES and a.size > share:
+            sys.stderr.write(f"dump-outputs: {name} is a seeded sample of {share} of its {a.size} elements\n")
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def workload_config(args):
@@ -306,28 +334,32 @@ def run_ours(args):
                         want=("rewards", "nll") if args.w_pg else ("nll",))
 
     def run_steps(first, n):
+        """Steps first .. first + n - 1 (batch i % pool, seed 0x5EED + i); returns the outputs of the last one."""
         if args.python_loop:
             for i in range(first, first + n):
                 b = devb[i % pool]
-                F.pg_ctc_step(b["logits"], b["targets"], b["in_len"], b["tgt_len"], K=K, seed=0x5EED + i,
-                              reward=args.reward, pg_weight=args.w_pg, ctc_weight=args.w_ctc,
-                              workspace=queue.workspace, want=("rewards", "nll") if args.w_pg else ("nll",))
-            return
+                out = F.pg_ctc_step(b["logits"], b["targets"], b["in_len"], b["tgt_len"], K=K, seed=0x5EED + i,
+                                    reward=args.reward, pg_weight=args.w_pg, ctc_weight=args.w_ctc,
+                                    workspace=queue.workspace, want=("rewards", "nll") if args.w_pg else ("nll",))
+            return {k: v for k, v in out.items() if isinstance(v, torch.Tensor)}
         done = 0
         while done < n:
             c = min(pool, n - done)
             queue.run(first=first + done, n=c, seed=0x5EED + first + done)
             done += c
+        return queue.outputs[(first + n - 1) % pool]
 
     # ---- device-resident throughput ("value") --------------------------------------------------
     # warm-up: at least W (>= 3) steps, and at least ~30 ms of them so that the SM clock has left its idle state before
-    # the timed region (a 20-step run is 1 ms of GPU time; the clocks line of the JSON shows what the timed region saw)
-    warm = max(args.warmup, 3)
+    # the timed region (a 20-step run is 1 ms of GPU time; the clocks line of the JSON shows what the timed region saw).
+    # The clock-driven part repeats steps first .. first + pool - 1, so the timed steps start at step `first` however
+    # long it ran: their batches and seeds, and so their outputs, depend on the arguments alone.
+    first = warm = max(args.warmup, 3)
     run_steps(0, warm)
     torch.cuda.synchronize()
     t_w = time.perf_counter()
     while time.perf_counter() - t_w < 0.03:
-        run_steps(warm, pool)
+        run_steps(first, pool)
         torch.cuda.synchronize()
         warm += pool
     D.barrier()
@@ -336,13 +368,15 @@ def run_ours(args):
     launches0 = _native.lib().pgasr_launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    run_steps(warm, args.steps)
+    last = run_steps(first, args.steps)
     e1.record()
     sampler.sample()
     torch.cuda.synchronize()
     sampler.sample()
     ms = D.max_over_ranks(e0.elapsed_time(e1))
     launches = _native.lib().pgasr_launch_count() - launches0
+    if args.dump_outputs and rank == 0:                  # before the steps below overwrite the queue's outputs
+        dump_outputs(args.dump_outputs, last)
     D.barrier()
     sampler.stop_flag = True
     sampler.join(1.0)

@@ -29,11 +29,12 @@ def _upstream():
     return mods["metrics"].edit_dist, mods["CTCdecoder"].collapse_fn
 
 
-def step(logits, targets, in_len, tgt_len, K, w_pg=1.0, w_ctc=1.0, seed=0):
-    """One PG + CTC loss step on the CPU.  Returns (loss, rewards [B,K], dlogits [B,T,V]) as numpy arrays."""
+def step(logits, targets, in_len, tgt_len, K, w_pg=1.0, w_ctc=1.0, seed=0, upstream=None):
+    """One PG + CTC loss step on the CPU.  Returns (loss, rewards [B,K], dlogits [B,T,V]) as numpy arrays.
+    `upstream`: the (edit_dist, collapse_fn) pair to run instead of the copies in oracle/_ref."""
     import numpy as np
     import torch
-    edit_dist, collapse_fn = _upstream()
+    edit_dist, collapse_fn = upstream or _upstream()
     z = torch.tensor(logits, dtype=torch.float32, requires_grad=True)
     B, T, V = z.shape
     logp_all = torch.log_softmax(z, dim=-1)

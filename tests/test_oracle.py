@@ -300,17 +300,19 @@ def test_togo_oracle_against_autograd(baseline_mode):
 
 
 def test_reference_cpu_leg_runs_on_upstream_code():
-    """oracle/refpath.py (the `kind: reference` CPU leg of bench.py) imports the REAL upstream collapse_fn / edit_dist
-    from oracle/_ref and agrees with the oracle on the CTC part (the sampled part differs by construction: torch RNG)."""
+    """oracle/refpath.py (the `kind: reference` CPU leg of bench.py) runs upstream's collapse_fn / edit_dist and agrees
+    with the oracle on the CTC part (the sampled part differs by construction: torch RNG).  Upstream's source is not
+    part of this repository: with no copy in oracle/_ref the leg runs oracle/pyref's restatements of the two
+    functions, which the golden vectors (upstream's own outputs) pin in test_edit_dist_golden and
+    test_evaluate_and_collapse_golden."""
     from oracle import make_ref, refpath
     make_ref.make()
-    if not refpath.available():
-        pytest.skip("no /root/reference here and oracle/_ref was not shipped")
+    upstream = None if refpath.available() else (pyref.edit_dist, pyref.collapse_fn)
     B, T, V, K, L = 2, 30, 6, 3, 4
     logits, targets, in_len, tgt_len, _ = make_batch(B, T, V, K, L, seed=5, ragged=True)
-    loss, R, g = refpath.step(logits, targets, in_len, tgt_len, K, w_pg=0.0, w_ctc=1.0)
+    loss, R, g = refpath.step(logits, targets, in_len, tgt_len, K, w_pg=0.0, w_ctc=1.0, upstream=upstream)
     nll, gref = cport.ctc_loss_grad(logits, targets, in_len, tgt_len)
     assert abs(loss - nll.mean()) < 1e-4 * abs(nll.mean())
     assert np.abs(g - gref / B).max() < 1e-5
-    loss, R, g = refpath.step(logits, targets, in_len, tgt_len, K, w_pg=1.0, w_ctc=0.0)
+    loss, R, g = refpath.step(logits, targets, in_len, tgt_len, K, w_pg=1.0, w_ctc=0.0, upstream=upstream)
     assert R.shape == (B, K) and (R <= 0).all() and np.isfinite(g).all()
