@@ -62,6 +62,13 @@ typedef enum {
  * r_i = -(ED(ref, hyp[:i+1]) - ED(ref, hyp[:i])) (policy_grad.py:10-15) credited to the frames that can still
  * influence them: reward-to-go G_t = sum over the symbols emitted at frames >= t (DESIGN.md "reward-to-go spec") */
 enum { PGASR_REWARD_NEG_ED = 0, PGASR_REWARD_NEG_CER = 1, PGASR_REWARD_ED_TO_GO = 2, PGASR_REWARD_MAX = 2 };
+/* word-level reward_mode (pgasr_pg_ctc_step_multi_ws only): R = -ED_w | R = -ED_w / n_w (the WER ratio of
+ * metrics.py:23-31), ED_w = Levenshtein distance between the WORD sequences of transcript and collapsed hypothesis,
+ * n_w = number of transcript words.  Words: the ids split at every occurrence of the separator id word_sep, exactly
+ * as Python's str.split(" ") splits a string (empty words kept: count(sep) + 1 words; the empty transcript is one
+ * empty word, so n_w >= 1).  Equals the upstream string split when every alphabet entry is one character
+ * (DESIGN.md "word reward spec").  PGASR_REWARD_MAX stays the bound of the entry points without word_sep. */
+enum { PGASR_REWARD_NEG_WED = 3, PGASR_REWARD_NEG_WER = 4 };
 /* baseline_mode: none | mean over the utterance's K samples | leave-one-out mean | external scalar */
 enum { PGASR_BASELINE_NONE = 0, PGASR_BASELINE_MEAN = 1, PGASR_BASELINE_LOO = 2, PGASR_BASELINE_VALUE = 3 };
 
@@ -95,6 +102,15 @@ PGASR_API int pgasr_collapse_u8(const uint8_t* seqs, const int32_t* seq_len, int
 PGASR_API int pgasr_edit_distance_u8(const uint8_t* hyps, const int32_t* hyp_len, int N, int hyp_stride,
                            const int32_t* refs, const int32_t* ref_len, int rows_per_ref,
                            int ref_stride, int vocab, int32_t* dist, int32_t* last_col, void* stream);
+/* ---- word edit distance: the same rows split into words at the separator id sep ---------------
+ * dist[r] = ED_w(refs[r / rows_per_ref, :ref_len], hyps[r, :hyp_len[r]]): Levenshtein distance over the word
+ * sequences (words compared by their ids; split semantics of PGASR_REWARD_NEG_WED), unit costs.
+ * ref_words (optional) [N / rows_per_ref] receives n_w = count(sep in ref) + 1 per reference: passed as the tgt_len
+ * of pgasr_pg_advantages with PGASR_REWARD_NEG_CER it gives the WER reward -ED_w / n_w.  ref_len <= 511
+ * (ref_stride <= 511), rows_per_ref <= 1024.  One CTA per reference, one warp per row.                         */
+PGASR_API int pgasr_word_edit_distance_u8(const uint8_t* hyps, const int32_t* hyp_len, int N, int hyp_stride,
+                                const int32_t* refs, const int32_t* ref_len, int rows_per_ref, int ref_stride,
+                                int sep, int32_t* dist, int32_t* ref_words, void* stream);
 PGASR_API int pgasr_edit_distance_i32(const int32_t* hyps, const int32_t* hyp_len, int N, int hyp_stride,
                             const int32_t* refs, const int32_t* ref_len, int rows_per_ref,
                             int ref_stride, int32_t* dist, void* stream);
@@ -187,6 +203,18 @@ PGASR_API int pgasr_pg_ctc_step_multi(const pgasr_step_io* steps, int n_steps, u
                             int B, int T, int V, int K, int Lmax, int blank,
                             int reward_mode, int baseline_mode, float baseline_value,
                             float w_pg, float w_ctc,
+                            void* workspace, size_t workspace_bytes, void* stream);
+/* The same with the word-level rewards: reward_mode may also be PGASR_REWARD_NEG_WED / _NEG_WER, word_sep is the id
+ * of the word separator (the space of the alphabet), in [0, V) and != blank (else PGASR_ERR_INVALID_ARG; it is
+ * checked, and ignored, for the character modes too).  The only entry point that takes the word modes; they are
+ * rejected everywhere else.  dist receives ED_w, hyp_len stays the length of the collapsed hypothesis in ids.  Same
+ * workspace (pgasr_pg_ctc_step_workspace_bytes) and kernel launches as the character modes: the single-launch kernel
+ * when its word-mode shared memory fits an SM, else the chain of stand-alone kernels with
+ * pgasr_word_edit_distance_u8.  Lmax <= 511.                                                                    */
+PGASR_API int pgasr_pg_ctc_step_multi_ws(const pgasr_step_io* steps, int n_steps, uint64_t seed_base,
+                            int B, int T, int V, int K, int Lmax, int blank,
+                            int reward_mode, int baseline_mode, float baseline_value,
+                            float w_pg, float w_ctc, int word_sep,
                             void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- CTC prefix beam search (upstream CTCdecoder.py:41-116, CTCDecoder.decode) -----------------------

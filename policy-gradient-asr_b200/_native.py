@@ -20,6 +20,7 @@ SIGNATURES = {
     "pgasr_softmax_sample": (_i, [_vp, _vp, _vp, _u64, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "pgasr_collapse_u8": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "pgasr_edit_distance_u8": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
+    "pgasr_word_edit_distance_u8": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "pgasr_edit_distance_i32": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _vp, _vp]),
     "pgasr_pg_advantages": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp, _vp, _vp, _vp]),
     "pgasr_pg_grad": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _i, _vp, _vp]),
@@ -32,6 +33,7 @@ SIGNATURES = {
     "pgasr_pg_ctc_step": (_i, [_vp, _vp, _vp, _vp, _vp, _u64, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f,
                                _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pgasr_pg_ctc_step_multi": (_i, [_vp, _i, _u64, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _vp, _sz, _vp]),
+    "pgasr_pg_ctc_step_multi_ws": (_i, [_vp, _i, _u64, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _i, _vp, _sz, _vp]),
     "pgasr_ctc_beam_search_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "pgasr_ctc_beam_search": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pgasr_host_create": (_i, [_i, _i, _i, _i, _i, _i, _vp]),

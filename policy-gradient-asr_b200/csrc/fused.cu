@@ -6,14 +6,15 @@
 
 #include "ctc_core.cuh"
 #include "fused_args.cuh"
+#include "words_core.cuh"
 
 namespace pgasr {
 
 constexpr int kFusedMaxK = 64;
-int launch_fused_spl4(int mode, FusedArgs& a, size_t smem, cudaStream_t st);
-int launch_fused_spl8(int mode, FusedArgs& a, size_t smem, cudaStream_t st);
-int launch_fused_spl16(int mode, FusedArgs& a, size_t smem, cudaStream_t st);
-int launch_fused_spl32(int mode, FusedArgs& a, size_t smem, cudaStream_t st);
+int launch_fused_spl4(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word);
+int launch_fused_spl8(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word);
+int launch_fused_spl16(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word);
+int launch_fused_spl32(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word);
 
 constexpr size_t kFusedSmemLimit = 220 * 1024;
 
@@ -82,6 +83,18 @@ static size_t pg_role_smem(int T, int V, int K, int spl, int threads, bool strea
     return pg;
 }
 
+// Word modes: the match tables have max(V, cap) + 1 rows (cap = word_class_cap), and the tail region holds
+// max(CDF rows, word-phase scratch): the scratch is used after P1, where the CDF rows are dead.
+static size_t pg_role_smem_word(int T, int V, int K, int Lmax, int spl, int threads, bool cdf, int nutt) {
+    const int W = spl / 2, cap = word_class_cap(Lmax, V), Vp = V > cap ? V : cap;
+    const size_t ub = W == 2 ? pg_u_bytes<2, 512>(T, Vp, K) : W == 4 ? pg_u_bytes<4, 512>(T, Vp, K) :
+                      W == 8 ? pg_u_bytes<8, 512>(T, Vp, K) : pg_u_bytes<16, 256>(T, Vp, K);
+    const size_t pg = (((size_t)T * V * 4 + 15) & ~(size_t)15) + (size_t)nutt * ub + 16;
+    const size_t scratch = word_tail_bytes(T, Lmax, cap, nutt, threads / 32);
+    const size_t cdfb = cdf ? pg_cdf_bytes(threads) : 0;
+    return pg + (cdfb > scratch ? cdfb : scratch);
+}
+
 // What the single-launch kernel can take for this shape.
 struct FusedPlan { int spl, threads; bool ctc_ok, gt, pg_ok, stream, bw; };
 
@@ -117,6 +130,12 @@ int fused_capability(int T, int V, int K, int Lmax) {
     return (pl.ctc_ok ? 1 : 0) | (pl.pg_ok ? 2 : 0);
 }
 
+bool fused_word_capability(int T, int V, int K, int Lmax) {
+    const FusedPlan pl = fused_plan(T, V, K, Lmax);
+    return pl.ctc_ok && pl.pg_ok && !pl.stream &&
+           pg_role_smem_word(T, V, K, Lmax, pl.spl, pl.threads, false, 1) <= kFusedSmemLimit;
+}
+
 // 0 when the fused kernel cannot take this shape at all (the caller then chains the stand-alone kernels)
 size_t fused_workspace_bytes(int B, int T, int V, int K, int Lmax) {
     const FusedPlan pl = fused_plan(T, V, K, Lmax);
@@ -125,7 +144,7 @@ size_t fused_workspace_bytes(int B, int T, int V, int K, int Lmax) {
 }
 
 // a.do_pg must be 0 when the PG role does not fit (fused_capability bit 1)
-int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput) {
+int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput, const WordArgs* word) {
     const FusedPlan pl = fused_plan(a.T, a.V, a.K, a.Lmax);
     if (!pl.ctc_ok || (a.do_pg && !pl.pg_ok)) return PGASR_ERR_UNSUPPORTED;
     const FusedWs w = fused_ws(a.B, a.T, a.V, pl.spl, pl.gt);
@@ -161,6 +180,25 @@ int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput) 
     // against 35.78 / 35.66).  Single steps keep it (back-to-back launches on one stream).  PGASR_PDL_THROUGHPUT=1: keep (A/B)
     static const bool pdl_tp = getenv("PGASR_PDL_THROUGHPUT") != nullptr;
     a.no_pdl = throughput && !pdl_tp;
+    if (!a.do_pg) word = nullptr;
+    if (word) {
+        // word modes: the same decisions as below on the word layout; the streaming PG role has no word phase
+        if (stream || !fused_word_capability(a.T, a.V, a.K, a.Lmax)) return PGASR_ERR_UNSUPPORTED;
+        static const bool no_pair = getenv("PGASR_NO_PAIR") != nullptr;
+        if (throughput && !no_pair && a.B >= 2 && a.V <= 32 &&
+            pg_role_smem_word(a.T, a.V, a.K, a.Lmax, pl.spl, pl.threads, true, 2) <= kFusedSmemLimit)
+            a.pg_pair = 1;
+        const int nutt = a.pg_pair ? 2 : 1;
+        size_t pg = pg_role_smem_word(a.T, a.V, a.K, a.Lmax, pl.spl, pl.threads, false, nutt);
+        if (pg > kFusedSmemLimit) return PGASR_ERR_UNSUPPORTED;
+        static const bool no_cdf = getenv("PGASR_NO_CDF_SMEM") != nullptr;
+        const size_t pg_cdf = pg_role_smem_word(a.T, a.V, a.K, a.Lmax, pl.spl, pl.threads, true, nutt);
+        if (!no_cdf && a.V <= 32 && pg_cdf <= kFusedSmemLimit) {
+            a.cdf_smem = 1;
+            pg = pg_cdf;
+        }
+        smem = smem > pg ? smem : pg;
+    } else
     if (a.do_pg) {
         // two utterances per PG CTA (their edit distances side by side) when the step is one of several in flight and both
         // blocks fit: measured 39.3 -> 36.5 us per step overlapped, but 58 -> 63 us for a step on its own (the pair CTA
@@ -181,10 +219,10 @@ int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput) 
     }
     const int mode = pl.bw ? 3 : !pl.gt ? 0 : !stream ? 1 : 2;   // tiles in shared memory | CTC streams | both stream | block workers
     switch (pl.spl) {
-        case 4: return launch_fused_spl4(mode, a, smem, st);
-        case 8: return launch_fused_spl8(mode, a, smem, st);
-        case 16: return launch_fused_spl16(mode, a, smem, st);
-        default: return launch_fused_spl32(mode, a, smem, st);
+        case 4: return launch_fused_spl4(mode, a, smem, st, word);
+        case 8: return launch_fused_spl8(mode, a, smem, st, word);
+        case 16: return launch_fused_spl16(mode, a, smem, st, word);
+        default: return launch_fused_spl32(mode, a, smem, st, word);
     }
 }
 

@@ -23,6 +23,13 @@ struct FusedArgs {
     float* tile_g;           // global-tile mode: [B][T + 2][RS] fp32 softmax rows (guard row before and after)
 };
 
+// Word-level rewards (reward_mode PGASR_REWARD_NEG_WED / _NEG_WER): a kernel argument of its own, next to FusedArgs, so
+// that the character-mode kernels keep their parameter block
+struct WordArgs {
+    int sep;                 // id of the word separator, in [0, V), != blank
+    int cap;                 // word_class_cap(Lmax, V): distinct transcript words a hypothesis can match
+};
+
 // shared-memory bytes of one utterance's block in a PG CTA (fused_impl.cuh: fused_pg_role; fused.cu sizes with it)
 template <int W, int kThreads>
 __host__ __device__ inline size_t pg_u_bytes(int T, int V, int K) {
@@ -41,7 +48,11 @@ size_t fused_workspace_bytes(int B, int T, int V, int K, int Lmax);
 // (armed once: the kernel re-arms it when it finishes)
 // throughput: the step is one of several independent ones in flight (pgasr_pg_ctc_step_multi): PG CTAs take two
 // utterances each -- less SM time per step, a longer single step; a step on its own keeps one utterance per PG CTA
-int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput = false);
+// word (non-NULL): the word-level rewards, a.do_pg set; the PG role must fit in its word layout (fused_word_capability)
+int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput = false, const WordArgs* word = nullptr);
+// the PG role of the word-level rewards fits an SM (logits tile in shared memory); otherwise the step chains the
+// stand-alone kernels for the PG part
+bool fused_word_capability(int T, int V, int K, int Lmax);
 size_t align256(size_t x);
 void fused_workspace_reset(const void* workspace, size_t bytes);   // forget the control-block parity of every fused workspace in the range
 

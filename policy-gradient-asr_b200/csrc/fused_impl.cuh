@@ -22,6 +22,7 @@
 #include "ctc_core.cuh"
 #include "fused_args.cuh"
 #include "myers_core.cuh"
+#include "words_core.cuh"
 
 namespace pgasr {
 
@@ -426,20 +427,30 @@ struct PgU {
     int *hlen_s, *dist_s;
     float* misc_s;
 };
-template <int W, int kThreads, bool kStream>
+// kWord (word-level rewards, DESIGN.md "word reward spec"): a word phase after P2 turns every collapsed hypothesis into
+// its sequence of word classes, the transcript's words become the match table, and P3 runs over words.
+// (the word arguments come as a parameter pack, empty for the character modes: their role keeps its exact signature --
+// where it is not inlined, an extra parameter changes its call frame)
+__device__ __forceinline__ WordArgs word_args_of() { return WordArgs{-1, 0}; }
+__device__ __forceinline__ WordArgs word_args_of(const WordArgs& w) { return w; }
+template <int W, int kThreads, bool kStream, bool kWord = false, typename... WA>
 __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned char* smem_raw, unsigned* s_last,
-                              unsigned long long* s_mbar) {
+                              unsigned long long* s_mbar, const WA&... word) {
+    static_assert(kWord == (sizeof...(WA) == 1), "the word modes take their WordArgs, the character modes none");
+    const WordArgs wa = word_args_of(word...);
     constexpr int kWarps = kThreads / 32;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int T = a.T, V = a.V, K = a.K;
     const int Tp = (T + 15) & ~15;
     const int Tp2 = (T / 2 + 16) & ~15;
+    // rows of the match tables: the alphabet, or (word modes) the transcript's word classes
+    const int Vp = kWord ? max(V, wa.cap) : V;
 
     // shared-memory carve-up: the logits tile (shared by the utterances of the CTA), one block per utterance, then the
     // reward-to-go arrays and the CDF rows
     float* ztile = reinterpret_cast<float*>(smem_raw);                                // [T][V] (tile mode only)
     const size_t off0 = kStream ? 0 : (((size_t)T * V * 4 + 15) & ~(size_t)15);
-    const size_t ubytes = pg_u_bytes<W, kThreads>(T, V, K);
+    const size_t ubytes = pg_u_bytes<W, kThreads>(T, Vp, K);
     auto pg_u = [&](int uu) {
         PgU X;
         X.b = b0 + uu;
@@ -452,15 +463,15 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
         X.samples_s = p + off;            off += (size_t)K * Tp;            // [K][Tp]
         X.hyp_s = p + off;                off += (size_t)K * Tp;            // [K][Tp]
         X.hrev_s = p + off;               off += (size_t)K * Tp2;           // [K][Tp2] second halves, reversed
-        X.peq = reinterpret_cast<uint32_t*>(p + off);   off += (size_t)(V + 1) * W * 4;
-        X.peq_r = reinterpret_cast<uint32_t*>(p + off); off += (size_t)(V + 1) * W * 4;   // reversed transcript
+        X.peq = reinterpret_cast<uint32_t*>(p + off);   off += (size_t)(Vp + 1) * W * 4;
+        X.peq_r = reinterpret_cast<uint32_t*>(p + off); off += (size_t)(Vp + 1) * W * 4;   // reversed transcript
         X.fg_s = reinterpret_cast<int16_t*>(p + off);   off += (size_t)((K + 7) & ~7) * (W * 32 + 2) * 2;   // (idle groups of the last warp get their own scratch)
         off = (off + 15) & ~(size_t)15;
         X.warp_acc = reinterpret_cast<double*>(p + off); off += (size_t)kWarps * kFusedMaxK * 8;   // log-prob partial sums
         X.adv_s = reinterpret_cast<float*>(p + off);     off += kFusedMaxK * 4;
         X.hlen_s = reinterpret_cast<int*>(p + off);      off += kFusedMaxK * 4;
         X.dist_s = reinterpret_cast<int*>(p + off);      off += kFusedMaxK * 4;
-        X.misc_s = reinterpret_cast<float*>(p + off);    // [0] sum of advantages
+        X.misc_s = reinterpret_cast<float*>(p + off);    // [0] sum of advantages; word modes: [1] n_w, [2] classes (int)
         return X;
     };
     size_t off = off0 + (size_t)nutt * ubytes;
@@ -473,6 +484,9 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
     int16_t* col_s = reinterpret_cast<int16_t*>(smem_raw + off); if (togo) off += (size_t)K * Tc * 2;   // [K][Tc]
     off = (off + 15) & ~(size_t)15;
     float* cdf_s = reinterpret_cast<float*>(smem_raw + off);     // [kThreads][33] (a.cdf_smem)
+    // word modes: the scratch of the word phase (transcripts, one block per warp) in place of the CDF rows, dead by then
+    unsigned char* const wtail = reinterpret_cast<unsigned char*>(cdf_s);
+    (void)wtail;
     unsigned nload = 0;                                    // bulk tile loads so far (the mbarrier's phase)
     int ref_rr[2][2];
 
@@ -511,7 +525,7 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
             ref_r[q] = j < m ? ref[j] : -1;
         }
         for (int i = threadIdx.x; i < kWarps * kFusedMaxK; i += kThreads) warp_acc[i] = 0.0;
-        for (int i = threadIdx.x; i < (V + 1) * W; i += kThreads) { peq[i] = 0u; peq_r[i] = 0u; }
+        for (int i = threadIdx.x; i < (Vp + 1) * W; i += kThreads) { peq[i] = 0u; peq_r[i] = 0u; }
         if (!kStream && a.bulk_tile) mbar_wait(s_mbar, nload++ & 1u);
         cp_async_wait<0>();
         __syncthreads();
@@ -717,6 +731,19 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
         (void)hlen_s; (void)dist_s; (void)misc_s; (void)lg; (void)ref; (void)Tb; (void)m;
         const int (&ref_r)[2] = ref_rr[uu];
         // ---- P2: collapse (one warp per sample) and the match table of the transcript ---------------
+        if constexpr (kWord) {
+            // word modes: the transcript as u8 ids for the word phase (0xFF: an id no hypothesis holds -- blank or
+            // outside [0, V) -- its word matches nothing), and that phase's zeroed hashes and flags
+            const WordRef R = word_ref_carve(wtail, uu, a.Lmax, wa.cap);
+            auto map_id = [&](int c) { return (uint8_t)((c >= 0 && c < V && c != a.blank) ? c : 0xFF); };
+#pragma unroll
+            for (int q = 0; q < 2; ++q) {
+                const int j = threadIdx.x + q * kThreads;
+                if (j < m) R.ref[j] = map_id(ref_r[q]);
+            }
+            for (int j = threadIdx.x + 2 * kThreads; j < m; j += kThreads) R.ref[j] = map_id(ref[j]);
+            for (int j = threadIdx.x; j < a.Lmax + 2; j += kThreads) { R.hash[j] = 0u; R.cls[j] = 0; }
+        } else {
 #pragma unroll
         for (int q = 0; q < 2; ++q) {
             const int j = threadIdx.x + q * kThreads;
@@ -735,6 +762,7 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
                 atomicOr(&peq_r[c * W + (jr >> 5)], 1u << (jr & 31));
             }
         }
+        }   // (character modes)
         for (int k = warp; k < K; k += kWarps) {
             const uint8_t* in = samples_s + (size_t)k * Tp;
             uint8_t* o = hyp_s + (size_t)k * Tp;
@@ -752,11 +780,118 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
             }
             if (lane == 0) hlen_s[k] = base;
             __syncwarp();
+            if constexpr (!kWord) {                           // (word modes: the word phase writes the halves)
             uint8_t* orv = hrev_s + (size_t)k * Tp2;          // the edit distance meets in the middle: second half backwards
             for (int i = lane; i < base / 2; i += 32) orv[i] = o[base - 1 - i];
+            }
         }
     }
     __syncthreads();
+
+    // ======== word phase (word modes): transcripts into word classes and match tables, hypotheses into class ids ========
+    if constexpr (kWord) {
+        PGASR_STAMP(b0 == 0 && threadIdx.x == 0, 61);
+        const unsigned lt = (1u << lane) - 1u;
+        // W1, warp uu for utterance uu: split the transcript (word_split_warp: ballot over the separators, hashes by
+        // shared-memory atomics), give every word whose ids a hypothesis can hold a class -- dense ids in the order of
+        // first occurrence, a word equal to an earlier one takes that one's class (hash and length filter, then id by
+        // id) -- and set its bit in the class's rows of the forward and the reversed match table
+        if (warp < nutt) {
+            const PgU X = pg_u(warp);
+            const WordRef R = word_ref_carve(wtail, warp, a.Lmax, wa.cap);
+            const int m = X.m;
+            const int nw = word_split_warp(R.ref, m, wa.sep, R.start, R.hash, R.cls);   // (R.cls: 1 = bad word)
+            if (lane == 0) R.start[0] = 0;
+            __syncwarp();
+            auto rlen = [&](int w) { return (w + 1 < nw ? (int)R.start[w + 1] - 1 : m) - (int)R.start[w]; };
+            for (int w = lane; w < nw; w += 32) R.key[w] = ((uint64_t)rlen(w) << 32) | R.hash[w];
+            __syncwarp();
+            int ncls = 0;
+            for (int w0 = 0; w0 < nw; w0 += 32) {
+                const int w = w0 + lane;
+                bool first = false;
+                int rep = w, s0 = 0;
+                uint64_t kw = 0u;
+                if (w < nw && R.cls[w] == 0) {                // (each lane reads and writes only its own word's flag)
+                    s0 = R.start[w]; kw = R.key[w];
+                    const int len = (int)(kw >> 32);
+                    first = true;
+                    // the first equal word (a bad one never is: it holds 0xFF): equal key, then equal ids
+                    for (int j = word_find_key(R.key, 0, w, kw); j < w; j = word_find_key(R.key, j + 1, w, kw)) {
+                        const int sj = R.start[j];
+                        bool eq = true;
+                        for (int i = 0; i < len && eq; ++i) eq = R.ref[sj + i] == R.ref[s0 + i];
+                        if (eq) { first = false; rep = j; break; }
+                    }
+                }
+                const unsigned fm = __ballot_sync(kFull, first);
+                const int c = ncls + __popc(fm & lt);
+                if (first) { R.cstart[c] = (uint16_t)s0; R.ckey[c] = kw; }
+                if (w < nw) { R.cls[w] = first ? (uint8_t)c : (uint8_t)0xFF; R.rep[w] = (uint16_t)rep; }
+                ncls += __popc(fm);
+            }
+            __syncwarp();
+            for (int w = lane; w < nw; w += 32) {             // repeated words: the class of their first occurrence
+                const int j = R.rep[w];
+                if (j != w) R.cls[w] = R.cls[j];
+            }
+            __syncwarp();
+            for (int w = lane; w < nw; w += 32) {
+                const uint32_t c = R.cls[w];
+                if (c != 0xFFu) {
+                    atomicOr(&X.peq[c * W + (w >> 5)], 1u << (w & 31));
+                    const int wr = nw - 1 - w;
+                    atomicOr(&X.peq_r[c * W + (wr >> 5)], 1u << (wr & 31));
+                }
+            }
+            if (lane == 0) { reinterpret_cast<int*>(X.misc_s)[1] = nw; reinterpret_cast<int*>(X.misc_s)[2] = ncls; }
+        }
+        __syncthreads();
+        PGASR_STAMP(b0 == 0 && threadIdx.x == 0, 62);
+        // W2, one warp per sample: split the collapsed hypothesis, look every word up among the transcript's classes
+        // (hash and length, then id by id; "absent" = the class count, the zero row of the tables), then write the class
+        // ids over the sample's characters -- forwards into hyp_s, the second half reversed into hrev_s -- for P3
+        {
+            const int tw = word_hyp_slots(T);
+            unsigned char* wp = wtail + (size_t)nutt * word_ref_bytes(a.Lmax, wa.cap) + (size_t)warp * word_warp_bytes(T);
+            uint16_t* hstart = reinterpret_cast<uint16_t*>(wp);
+            uint32_t* hhash = reinterpret_cast<uint32_t*>(wp + word_a16(2 * (size_t)tw));
+            uint8_t* hid = wp + word_a16(2 * (size_t)tw) + 4 * (size_t)tw;
+            for (int sidx = warp; sidx < nutt * K; sidx += kWarps) {
+                const int uu = sidx / K, k = sidx - uu * K;
+                const PgU X = pg_u(uu);
+                const WordRef R = word_ref_carve(wtail, uu, a.Lmax, wa.cap);
+                const int ncls = reinterpret_cast<const int*>(X.misc_s)[2];
+                const int n = X.hlen_s[k];
+                uint8_t* row = X.hyp_s + (size_t)k * Tp;
+                for (int i = lane; i < tw; i += 32) hhash[i] = 0u;
+                __syncwarp();
+                const int nwh = word_split_warp(row, n, wa.sep, hstart, hhash, nullptr);
+                if (lane == 0) hstart[0] = 0;
+                __syncwarp();
+                for (int w = lane; w < nwh; w += 32) {
+                    const int s0 = hstart[w], len = (w + 1 < nwh ? (int)hstart[w + 1] - 1 : n) - s0;
+                    const uint64_t kw = ((uint64_t)len << 32) | hhash[w];
+                    int id = ncls;
+                    for (int c = word_find_key(R.ckey, 0, ncls, kw); c < ncls; c = word_find_key(R.ckey, c + 1, ncls, kw)) {
+                        const int cs = R.cstart[c];
+                        bool eq = true;
+                        for (int i = 0; i < len && eq; ++i) eq = R.ref[cs + i] == row[s0 + i];
+                        if (eq) { id = c; break; }
+                    }
+                    hid[w] = (uint8_t)id;
+                }
+                __syncwarp();                                 // (every lane is done reading the characters)
+                for (int i = lane; i < nwh; i += 32) row[i] = hid[i];
+                const int n1 = myers_split_point(nwh);
+                uint8_t* rv = X.hrev_s + (size_t)k * Tp2;
+                for (int i = lane; i < nwh - n1; i += 32) rv[i] = hid[nwh - 1 - i];
+                if (lane == 0) X.dist_s[k] = nwh;             // (P3 reads the word count here, then writes the distance)
+                __syncwarp();
+            }
+        }
+        __syncthreads();
+    }
 
     PGASR_STAMP(b0 == 0 && threadIdx.x == 0, 33);
     // ======== edit distances: the utterances of the CTA side by side ========
@@ -849,25 +984,26 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
                 const int tid = (wl - (fwd ? 0 : nw)) * 32 + lane;
                 k = tid / P; p = tid % P;
                 const int kc = min(k, K - 1);
-                n = k < K ? X.hlen_s[kc] : 0;
+                n = k < K ? (kWord ? X.dist_s : X.hlen_s)[kc] : 0;
                 n1 = bidir ? myers_split_point(n) : n;
                 const int nsym = fwd ? n1 : n - n1;
                 const int nmax = __reduce_max_sync(kFull, nsym);
                 myers_half<W, P, false>(fwd ? X.hyp_s + (size_t)kc * Tp : X.hrev_s + (size_t)kc * Tp2, nsym, fwd ? X.peq : X.peq_r,
-                                        V, p, nmax, VPh, VNh);
+                                        kWord ? reinterpret_cast<const int*>(X.misc_s)[2] : V, p, nmax, VPh, VNh);
                 if (!fwd) myers_store_column<W, P>(VPh, VNh, n - n1, p, X.fg_s + (size_t)k * (W * 32 + 2));
             }
             __syncthreads();
             if (mine && wl < nw) {
+                const int mq = kWord ? reinterpret_cast<const int*>(X.misc_s)[1] : X.m;   // (word modes: n_w)
                 int d;
                 if (bidir) {
-                    d = myers_meet<W, P>(VPh, VNh, n1, X.m, p, X.fg_s + (size_t)k * (W * 32 + 2));
+                    d = myers_meet<W, P>(VPh, VNh, n1, mq, p, X.fg_s + (size_t)k * (W * 32 + 2));
                 } else {                                  // dp[n, m] = n + sum_{j<m} (VP_j - VN_j)
                     d = 0;
 #pragma unroll
                     for (int w = 0; w < W / P; ++w) {
                         const int lo = (p * (W / P) + w) * 32;
-                        const uint32_t msk = X.m >= lo + 32 ? 0xffffffffu : (X.m > lo ? (1u << (X.m - lo)) - 1u : 0u);
+                        const uint32_t msk = mq >= lo + 32 ? 0xffffffffu : (mq > lo ? (1u << (mq - lo)) - 1u : 0u);
                         d += __popc(VPh[w] & msk) - __popc(VNh[w] & msk);
                     }
 #pragma unroll
@@ -881,6 +1017,10 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
         if ((int)threadIdx.x < nutt * K) {
             const PgU X = pg_u((int)threadIdx.x / K);
             const int k = (int)threadIdx.x % K;
+            if constexpr (kWord) {
+                const int* wi = reinterpret_cast<const int*>(X.misc_s);
+                X.dist_s[k] = myers_row<W, false>(X.hyp_s + (size_t)k * Tp, X.dist_s[k], X.peq, wi[2], wi[1], static_cast<int32_t*>(nullptr));
+            } else
             X.dist_s[k] = myers_row<W, false>(X.hyp_s + (size_t)k * Tp, X.hlen_s[k], X.peq, V, X.m, static_cast<int32_t*>(nullptr));
         }
     }
@@ -909,6 +1049,9 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
             for (int k = lane; k < K; k += 32) {
                 float R = -(float)dist_s[k];
                 if (a.reward_mode == PGASR_REWARD_NEG_CER) R = __fdiv_rn(R, (float)m);
+                if constexpr (kWord) {                        // -ED_w / n_w, the WER ratio
+                    if (a.reward_mode == PGASR_REWARD_NEG_WER) R = __fdiv_rn(R, (float)reinterpret_cast<const int*>(misc_s)[1]);
+                }
                 if (togo) R = (float)(m - dist_s[k]);         // G_0 = c[0] - c[n]: what the whole hypothesis earned
                 adv_s[k] = R;
                 sumR += (double)R;
@@ -1197,16 +1340,60 @@ __global__ void __launch_bounds__(kThreads, 1) pg_ctc_fused_kernel(const FusedAr
 #endif
 }
 
-template <int SPL, int kThreads, bool kGT, bool kStream, bool kBW = false>
-static int launch_fused(FusedArgs& a, size_t smem, cudaStream_t st) {
-    // the opt-in is sticky PER DEVICE: raise it only when a larger tile comes on the device the launch goes to
-    static thread_local size_t smem_set[64] = {0};
+// word-level rewards (tile mode: the PG role keeps the logits tile in shared memory): the kernel above with the word
+// phase in its PG role (fused_pg_role<..., true>); same ticket protocol, no timing stamps
+template <int SPL, int kThreads, bool kGT, bool kBW>
+__global__ void __launch_bounds__(kThreads, 1) pg_ctc_fused_word_kernel(const FusedArgs a, const WordArgs wa) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ unsigned s_ticket, s_last;
+    __shared__ __align__(8) unsigned long long s_mbar;
+    if (threadIdx.x == 0 && a.bulk_tile) {
+        mbar_init(&s_mbar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    }
+    if (threadIdx.x == 0) s_ticket = atomicAdd(a.ctrl, 1u);
+    __syncthreads();
+    asm volatile("griddepcontrol.wait;\n" ::: "memory");
+    asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory");
+    const unsigned ticket = s_ticket;
+    const unsigned n_ctc = a.do_ctc ? (unsigned)a.B : 0u;
+    if (ticket < n_ctc) fused_ctc_role<SPL, kThreads, kGT, kBW>(a, (int)ticket, smem_raw, &s_last, &s_mbar);
+    else {
+        const int j = (int)(ticket - n_ctc);
+        const int b0 = a.pg_pair ? 2 * j : j;
+        fused_pg_role<SPL / 2, kThreads, false, true>(a, b0, a.pg_pair ? min(2, a.B - b0) : 1, smem_raw, &s_last, &s_mbar,
+                                                      wa);
+    }
+    __syncthreads();
+    if (s_last && threadIdx.x < 32 && ticket < n_ctc) loss_reduce_and_rearm(a);
+}
+
+// the dynamic shared-memory opt-in of `kern`: sticky PER DEVICE, raised only when a larger tile comes on the device the
+// launch goes to (smem_set: one per kernel)
+template <typename Kern>
+static int fused_smem_optin(Kern kern, size_t (&smem_set)[64], size_t smem) {
     int dev = 0;
     PGASR_CUDA_TRY(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64 || smem > smem_set[dev]) {
-        PGASR_CUDA_TRY(cudaFuncSetAttribute(pg_ctc_fused_kernel<SPL, kThreads, kGT, kStream, kBW>,
-                                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        PGASR_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         if (dev >= 0 && dev < 64) smem_set[dev] = smem;
+    }
+    return PGASR_OK;
+}
+
+template <int SPL, int kThreads, bool kGT, bool kStream, bool kBW = false>
+static int launch_fused(FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word = nullptr) {
+    static thread_local size_t smem_set[64] = {0};
+    static thread_local size_t smem_set_w[64] = {0};
+    if constexpr (!kStream) {
+        if (word) {
+            const int rc = fused_smem_optin(pg_ctc_fused_word_kernel<SPL, kThreads, kGT, kBW>, smem_set_w, smem);
+            if (rc) return rc;
+        }
+    }
+    if (!word) {
+        const int rc = fused_smem_optin(pg_ctc_fused_kernel<SPL, kThreads, kGT, kStream, kBW>, smem_set, smem);
+        if (rc) return rc;
     }
     const int grid = (a.do_ctc ? a.B : 0) + (a.do_pg ? (a.pg_pair ? (a.B + 1) / 2 : a.B) : 0);
     static const bool no_pdl = getenv("PGASR_NO_PDL") != nullptr;     // (A/B measurements)
@@ -1220,6 +1407,14 @@ static int launch_fused(FusedArgs& a, size_t smem, cudaStream_t st) {
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = (no_pdl || a.no_pdl) ? 0 : 1;
+    if constexpr (!kStream) {
+        if (word) {
+            PGASR_CUDA_TRY(cudaLaunchKernelEx(&cfg, pg_ctc_fused_word_kernel<SPL, kThreads, kGT, kBW>, a, *word));
+            ++g_launches;
+            return PGASR_OK;
+        }
+    }
+    if (word) return PGASR_ERR_UNSUPPORTED;
     PGASR_CUDA_TRY(cudaLaunchKernelEx(&cfg, pg_ctc_fused_kernel<SPL, kThreads, kGT, kStream, kBW>, a));
     ++g_launches;
     return PGASR_OK;
@@ -1228,15 +1423,16 @@ static int launch_fused(FusedArgs& a, size_t smem, cudaStream_t st) {
 // one translation unit per SPL instantiates its modes (0: tiles in shared memory, 1: the CTC role streams,
 // 2: both roles stream, 3: tiles in shared memory with block workers -- up to 8 states per lane only) so that the
 // variants compile in parallel
+// word (non-NULL): the word-mode kernel, modes 0, 1 and 3 (the PG role keeps its tile in shared memory)
 template <int SPL, int kThreads>
-int launch_fused_modes(int mode, FusedArgs& a, size_t smem, cudaStream_t st) {
+int launch_fused_modes(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word) {
     if constexpr (SPL <= 8) {
-        if (mode == 3) return launch_fused<SPL, kThreads, false, false, true>(a, smem, st);
+        if (mode == 3) return launch_fused<SPL, kThreads, false, false, true>(a, smem, st, word);
     }
     switch (mode) {
-        case 0: return launch_fused<SPL, kThreads, false, false>(a, smem, st);
-        case 1: return launch_fused<SPL, kThreads, true, false>(a, smem, st);
-        default: return launch_fused<SPL, kThreads, true, true>(a, smem, st);
+        case 0: return launch_fused<SPL, kThreads, false, false>(a, smem, st, word);
+        case 1: return launch_fused<SPL, kThreads, true, false>(a, smem, st, word);
+        default: return launch_fused<SPL, kThreads, true, true>(a, smem, st, word);
     }
 }
 

@@ -2,8 +2,8 @@
 #include "fused_impl.cuh"
 
 namespace pgasr {
-int launch_fused_spl8(int mode, FusedArgs& a, size_t smem, cudaStream_t st) {
-    return launch_fused_modes<8, 512>(mode, a, smem, st);
+int launch_fused_spl8(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word) {
+    return launch_fused_modes<8, 512>(mode, a, smem, st, word);
 }
 }  // namespace pgasr
 

@@ -3,6 +3,7 @@
 #include <cstdlib>
 
 #include "fused_args.cuh"
+#include "words_core.cuh"
 
 namespace pgasr {
 
@@ -149,12 +150,20 @@ namespace pgasr {
 struct StepParams {
     int B, T, V, K, Lmax, blank, reward_mode, baseline_mode;
     float baseline_value, w_pg, w_ctc;
+    int word_sep;            // -1: entry points without word modes (reward_mode <= PGASR_REWARD_MAX)
 };
+
+static bool word_mode(int reward_mode) {
+    return reward_mode == PGASR_REWARD_NEG_WED || reward_mode == PGASR_REWARD_NEG_WER;
+}
 
 static int step_check(const StepParams& q, const void* workspace, size_t workspace_bytes) {
     if (!workspace || q.B <= 0 || q.T <= 0 || q.V <= 0 || q.K <= 0 || q.Lmax <= 0 || q.blank < 0 || q.blank >= q.V)
         return PGASR_ERR_INVALID_ARG;
-    if (q.reward_mode < 0 || q.reward_mode > PGASR_REWARD_MAX || q.baseline_mode < 0 || q.baseline_mode > 3)
+    const bool words = q.word_sep >= 0 && q.word_sep < q.V && q.word_sep != q.blank;
+    if (q.word_sep != -1 && !words) return PGASR_ERR_INVALID_ARG;   // (pgasr_pg_ctc_step_multi_ws: the separator)
+    if (q.reward_mode < 0 || (q.reward_mode > PGASR_REWARD_MAX && !(words && word_mode(q.reward_mode))) ||
+        q.baseline_mode < 0 || q.baseline_mode > 3)
         return PGASR_ERR_INVALID_ARG;
     if (q.K > 64 || q.V > kMaxV) return PGASR_ERR_UNSUPPORTED;
     const size_t need = pgasr_pg_ctc_step_workspace_bytes(q.B, q.T, q.V, q.K, q.Lmax);
@@ -172,6 +181,10 @@ static int step_one(const StepParams& q, const pgasr_step_io& io, uint64_t seed,
     const int B = q.B, T = q.T, V = q.V, K = q.K, Lmax = q.Lmax;
     const bool do_pg = q.w_pg != 0.0f, do_ctc = q.w_ctc != 0.0f;
     const int cap = step_fused_capability(B, T, V, K, Lmax);
+    const bool words = word_mode(q.reward_mode);
+    // word modes: the single-launch kernel when its word layout fits, else the PG part chains the stand-alone kernels
+    const bool words_fused = words && do_pg && fused_word_capability(T, V, K, Lmax);
+    const WordArgs wa = {q.word_sep, word_class_cap(Lmax, V)};
     FusedArgs a;
     a.logits = io.logits; a.targets = io.targets; a.in_len = io.in_len; a.tgt_len = io.tgt_len; a.uniforms = io.uniforms;
     a.seed = seed; a.B = B; a.T = T; a.V = V; a.K = K; a.Lmax = Lmax; a.blank = q.blank;
@@ -179,9 +192,9 @@ static int step_one(const StepParams& q, const pgasr_step_io& io, uint64_t seed,
     a.w_pg = q.w_pg; a.w_ctc = q.w_ctc; a.do_pg = do_pg; a.do_ctc = do_ctc;
     a.loss = io.loss; a.dlogits = io.dlogits; a.rewards = io.rewards; a.logp = io.logp; a.hyp_len = io.hyp_len;
     a.dist = io.dist; a.nll = io.nll; a.samples = io.samples; a.to_go = io.to_go; a.r_pos = io.r_pos;
-    if ((do_pg || do_ctc) && (cap & 1) && (!do_pg || (cap & 2))) {
+    if ((do_pg || do_ctc) && (cap & 1) && (!do_pg || (cap & 2)) && (!words || !do_pg || words_fused)) {
         // one launch: heterogeneous CTAs (CTC role / PG role per utterance), see fused.cu
-        return fused_step(a, workspace, st, throughput);
+        return fused_step(a, workspace, st, throughput, words && do_pg ? &wa : nullptr);
     }
     if (do_pg && q.reward_mode == PGASR_REWARD_ED_TO_GO) return PGASR_ERR_UNSUPPORTED;   // (single-launch kernel only)
     // long utterances: the PG role's tiles do not fit one SM -- the PG part runs as the chain of stand-alone
@@ -205,11 +218,24 @@ static int step_one(const StepParams& q, const pgasr_step_io& io, uint64_t seed,
     if (do_pg) {
         rc = pgasr_collapse_u8(smp, io.in_len, K, B * K, T, q.blank, w.hyps, hl, stream);
         if (rc) return rc;
+        if (words) {
+            // word counts of the transcripts in the stand-alone nll scratch: unused when the caller takes nll, else first
+            // written by the CTC part below, after the advantages have read them.  They are the lengths of the WER ratio.
+            int32_t* nw = reinterpret_cast<int32_t*>(w.nll);
+            rc = pgasr_word_edit_distance_u8(w.hyps, hl, B * K, T, io.targets, io.tgt_len, K, Lmax, q.word_sep, ds, nw,
+                                             stream);
+            if (rc) return rc;
+            rc = pgasr_pg_advantages(ds, nw, lp, B, K, Lmax,
+                                     q.reward_mode == PGASR_REWARD_NEG_WER ? PGASR_REWARD_NEG_CER : PGASR_REWARD_NEG_ED,
+                                     q.baseline_mode, q.baseline_value, rw, w.adv, w.loss_terms, stream);
+            if (rc) return rc;
+        } else {
         rc = pgasr_edit_distance_u8(w.hyps, hl, B * K, T, io.targets, io.tgt_len, K, Lmax, V, ds, nullptr, stream);
         if (rc) return rc;
         rc = pgasr_pg_advantages(ds, io.tgt_len, lp, B, K, Lmax, q.reward_mode, q.baseline_mode, q.baseline_value, rw,
                                  w.adv, w.loss_terms, stream);
         if (rc) return rc;
+        }
     }
     if (do_ctc && (cap & 1)) {
         a.do_pg = 0; a.rewards = nullptr; a.logp = nullptr; a.hyp_len = nullptr; a.dist = nullptr; a.samples = nullptr;
@@ -242,7 +268,7 @@ extern "C" int pgasr_pg_ctc_step(const float* logits, const int32_t* targets, co
                                  float* rewards, float* logp, int32_t* hyp_len, int32_t* dist, float* nll,
                                  uint8_t* samples, void* workspace, size_t workspace_bytes, void* stream) {
     using namespace pgasr;
-    const StepParams q = {B, T, V, K, Lmax, blank, reward_mode, baseline_mode, baseline_value, w_pg, w_ctc};
+    const StepParams q = {B, T, V, K, Lmax, blank, reward_mode, baseline_mode, baseline_value, w_pg, w_ctc, -1};
     if (!logits || !targets || !loss || !dlogits) return PGASR_ERR_INVALID_ARG;
     const int rc = step_check(q, workspace, workspace_bytes);
     if (rc) return rc;
@@ -284,12 +310,35 @@ static int aux_lane(AuxLane** out) {
 // at the headline shape) and its tail -- while steps three apart stay ordered (same stream; programmatic dependent
 // launch overlaps their launch latency).  The extra streams are forked from and joined back into `stream` with
 // events, so to the caller the call is ordered on `stream` like any other.  PGASR_NO_OVERLAP=1: one stream.
+namespace pgasr {
+static int step_multi(const StepParams& q, const pgasr_step_io* steps, int n_steps, uint64_t seed_base,
+                      void* workspace, size_t workspace_bytes, void* stream);
+}
+
 extern "C" int pgasr_pg_ctc_step_multi(const pgasr_step_io* steps, int n_steps, uint64_t seed_base, int B, int T,
                                        int V, int K, int Lmax, int blank, int reward_mode, int baseline_mode,
                                        float baseline_value, float w_pg, float w_ctc, void* workspace,
                                        size_t workspace_bytes, void* stream) {
     using namespace pgasr;
-    const StepParams q = {B, T, V, K, Lmax, blank, reward_mode, baseline_mode, baseline_value, w_pg, w_ctc};
+    const StepParams q = {B, T, V, K, Lmax, blank, reward_mode, baseline_mode, baseline_value, w_pg, w_ctc, -1};
+    return step_multi(q, steps, n_steps, seed_base, workspace, workspace_bytes, stream);
+}
+
+// the same with the word-level rewards (word_sep: the separator id; checked for every mode)
+extern "C" int pgasr_pg_ctc_step_multi_ws(const pgasr_step_io* steps, int n_steps, uint64_t seed_base, int B, int T,
+                                          int V, int K, int Lmax, int blank, int reward_mode, int baseline_mode,
+                                          float baseline_value, float w_pg, float w_ctc, int word_sep, void* workspace,
+                                          size_t workspace_bytes, void* stream) {
+    using namespace pgasr;
+    if (word_sep < 0 || word_sep >= V || word_sep == blank) return PGASR_ERR_INVALID_ARG;
+    const StepParams q = {B, T, V, K, Lmax, blank, reward_mode, baseline_mode, baseline_value, w_pg, w_ctc, word_sep};
+    return step_multi(q, steps, n_steps, seed_base, workspace, workspace_bytes, stream);
+}
+
+namespace pgasr {
+static int step_multi(const StepParams& q, const pgasr_step_io* steps, int n_steps, uint64_t seed_base,
+                      void* workspace, size_t workspace_bytes, void* stream) {
+    const int B = q.B, T = q.T, V = q.V, K = q.K, Lmax = q.Lmax;
     if (!steps || n_steps < 0) return PGASR_ERR_INVALID_ARG;
     int rc = step_check(q, workspace, workspace_bytes);
     if (rc) return rc;
@@ -316,3 +365,4 @@ extern "C" int pgasr_pg_ctc_step_multi(const pgasr_step_io* steps, int n_steps, 
     }
     return rc;
 }
+}  // namespace pgasr

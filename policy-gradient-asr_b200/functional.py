@@ -10,7 +10,8 @@ import torch
 
 from . import _native
 
-REWARD_MODES = {"ed": 0, "cer": 1, "ed_to_go": 2}
+REWARD_MODES = {"ed": 0, "cer": 1, "ed_to_go": 2, "wed": 3, "wer": 4}
+WORD_REWARDS = ("wed", "wer")      # word-level: need the separator id (space_id), pgasr_pg_ctc_step_multi_ws
 NO_IGNORE = -2**31                  # PGASR_NO_IGNORE
 OPTIONAL_OUTPUTS = ("rewards", "logp", "hyp_len", "dist", "nll", "samples", "to_go", "r_pos")
 BASELINE_MODES = {"none": 0, "mean": 1, "loo": 2, "value": 3}
@@ -126,6 +127,30 @@ def edit_distance(hyps, hyp_len, refs, ref_len=None, rows_per_ref=None, vocab=25
                  rows_per_ref, Lr, int(vocab), _ptr(dist), _ptr(col))
     dist = dist.reshape(shape[:-1])
     return (dist, col.reshape(*shape[:-1], Th + 1)) if last_col else dist
+
+
+def word_edit_distance(hyps, hyp_len, refs, sep, ref_len=None, rows_per_ref=None):
+    """Word-level rows a1/a4: hyps [N,Th] (or [B,K,Th]) uint8, refs [G,Lr] int32, both split into words at the id
+    `sep` (str.split(" ") semantics: empty words kept) -> (dist [N] int32 word edit distances, ref_words [G] int32 =
+    words per reference).  len(ref) <= 511."""
+    hyps = _need(hyps, torch.uint8, "hyps")
+    shape = hyps.shape
+    Th = shape[-1]
+    flat = hyps.reshape(-1, Th)
+    N = flat.shape[0]
+    refs = _need(refs, torch.int32, "refs", 2)
+    G, Lr = refs.shape
+    if rows_per_ref is None:
+        rows_per_ref = N // max(G, 1)
+    if G * rows_per_ref != N:
+        raise ValueError("hyps rows must be refs rows * rows_per_ref")
+    hyp_len = _opt_i32(hyp_len, "hyp_len", N, hyps.device)
+    ref_len = _opt_i32(ref_len, "ref_len", G, hyps.device)
+    dist = torch.empty((N,), dtype=torch.int32, device=hyps.device)
+    ref_words = torch.empty((G,), dtype=torch.int32, device=hyps.device)
+    _launch(hyps, "pgasr_word_edit_distance_u8", _ptr(flat), _ptr(hyp_len), N, Th, _ptr(refs), _ptr(ref_len),
+            rows_per_ref, Lr, int(sep), _ptr(dist), _ptr(ref_words))
+    return dist.reshape(shape[:-1]), ref_words
 
 
 def edit_distance_tokens(hyps, hyp_len, refs, ref_len=None, rows_per_ref=1):
@@ -326,13 +351,30 @@ def _prep_batch(logits, targets, input_lengths, target_lengths, uniforms, K):
     return batch, (B, T, V, int(K), Lmax), dev
 
 
+def _step_entry(reward, blank, space_id):
+    """(entry point name, extra arguments before the workspace): the word rewards go through
+    pgasr_pg_ctc_step_multi_ws with the separator id, every other mode through pgasr_pg_ctc_step_multi."""
+    if reward not in REWARD_MODES:
+        raise ValueError(f"unknown reward {reward!r}; choose from {tuple(REWARD_MODES)}")
+    if reward not in WORD_REWARDS:
+        return "pgasr_pg_ctc_step_multi", ()
+    if space_id is None:
+        raise ValueError(f"reward={reward!r} needs space_id, the id of the word separator (the space character)")
+    if int(space_id) == int(blank):
+        raise ValueError("space_id must differ from blank")
+    return "pgasr_pg_ctc_step_multi_ws", (int(space_id),)
+
+
 def pg_ctc_step(logits, targets, input_lengths=None, target_lengths=None, K=16, blank=0, reward="ed",
                 baseline="mean", baseline_value=0.0, pg_weight=1.0, ctc_weight=1.0, uniforms=None, seed=0,
-                workspace=None, want=("rewards", "nll"), out=None):
+                workspace=None, want=("rewards", "nll"), out=None, space_id=None):
     """The whole loss step (rows a1-a8 chained) in one C-ABI call.
     Returns a dict: loss (0-d), dlogits [B,T,V], plus the optional outputs named in `want` out of
     rewards, logp, hyp_len, dist, nll, samples (and, with reward='ed_to_go', to_go and r_pos [B,K,T]).
-    `out`: a dict from StepWorkspace.outputs() to write into instead of allocating (no allocation per step)."""
+    `out`: a dict from StepWorkspace.outputs() to write into instead of allocating (no allocation per step).
+    reward='wed' / 'wer' (word edit distance, -WED / n_words): space_id is the id of the word separator; dist then
+    holds word edit distances (hyp_len stays in ids)."""
+    entry, extra = _step_entry(reward, blank, space_id)
     batch, key, dev = _prep_batch(logits, targets, input_lengths, target_lengths, uniforms, K)
     B, T, V, K, Lmax = key
     if workspace is None or workspace.key != key or workspace.device != dev:
@@ -342,8 +384,8 @@ def pg_ctc_step(logits, targets, input_lengths=None, target_lengths=None, K=16, 
     else:
         _check_outputs(out, key, dev)
     io = _step_io(batch, out, seed)
-    _launch(logits, "pgasr_pg_ctc_step_multi", C.byref(io), 1, 0, B, T, V, K, Lmax, int(blank), REWARD_MODES[reward],
-            BASELINE_MODES[baseline], float(baseline_value), float(pg_weight), float(ctc_weight),
+    _launch(logits, entry, C.byref(io), 1, 0, B, T, V, K, Lmax, int(blank), REWARD_MODES[reward],
+            BASELINE_MODES[baseline], float(baseline_value), float(pg_weight), float(ctc_weight), *extra,
             _ptr(workspace.buf), workspace.nbytes)
     res = dict(out)
     res["loss"] = out["loss"][0]
@@ -361,7 +403,8 @@ class StepQueue:
     """
 
     def __init__(self, batches, K=16, blank=0, reward="ed", baseline="mean", baseline_value=0.0, pg_weight=1.0,
-                 ctc_weight=1.0, want=("rewards", "nll"), workspace=None):
+                 ctc_weight=1.0, want=("rewards", "nll"), workspace=None, space_id=None):
+        self._entry, self._extra = _step_entry(reward, blank, space_id)
         if not batches:
             raise ValueError("StepQueue needs at least one batch")
         self.batches, self.outputs = [], []
@@ -397,6 +440,6 @@ class StepQueue:
         first = int(first) % nb
         B, T, V, K, Lmax = self.key
         base = C.addressof(self._io) + first * self._stride
-        _launch(self.workspace.buf, "pgasr_pg_ctc_step_multi", base, n, (int(seed) - first) & (2**64 - 1), B, T, V, K,
-                Lmax, *self.params, _ptr(self.workspace.buf), self.workspace.nbytes)
+        _launch(self.workspace.buf, self._entry, base, n, (int(seed) - first) & (2**64 - 1), B, T, V, K,
+                Lmax, *self.params, *self._extra, _ptr(self.workspace.buf), self.workspace.nbytes)
         return n

@@ -17,7 +17,7 @@ import ctypes as C
 import torch
 
 from . import _native
-from .functional import BASELINE_MODES, REWARD_MODES
+from .functional import BASELINE_MODES, REWARD_MODES, WORD_REWARDS
 
 
 def _host(t, dtype, name, numel=None, optional=False):
@@ -41,6 +41,9 @@ def _host(t, dtype, name, numel=None, optional=False):
 class HostPipeline:
     def __init__(self, B, T, V, K, Lmax, depth=3, blank=0, reward="ed", baseline="mean", baseline_value=0.0,
                  pg_weight=1.0, ctc_weight=1.0):
+        if reward in WORD_REWARDS:
+            raise ValueError(f"reward={reward!r} (word level) is not available on host buffers; use "
+                             "functional.pg_ctc_step or PolicyGradCTCLoss with device tensors")
         self.shape = (int(B), int(T), int(V), int(K), int(Lmax))
         self.depth = int(depth)
         self.blank, self.reward, self.baseline = int(blank), REWARD_MODES[reward], BASELINE_MODES[baseline]

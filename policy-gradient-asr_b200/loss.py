@@ -48,6 +48,7 @@ class _PGCTCFn(torch.autograd.Function):
                             blank=module.blank, reward=module.reward, baseline=module.baseline,
                             baseline_value=module.baseline_value, pg_weight=module.pg_weight,
                             ctc_weight=module.ctc_weight, uniforms=uniforms, seed=module._next_seed(),
+                            space_id=module.space_id,
                             workspace=module._workspace, want=("rewards", "nll", "logp", "dist", "hyp_len"))
         module._workspace = out["workspace"]
         module.last = {k: out[k] for k in ("rewards", "nll", "logp", "dist", "hyp_len")}
@@ -67,18 +68,29 @@ class PolicyGradCTCLoss(nn.Module):
             uniforms[B,K,T]=None) -> 0-d tensor attached to `logits`.
     reward: 'ed' (-edit distance), 'cer' (-edit distance / len(transcript), as metrics.evaluate's CER) or
             'ed_to_go' (upstream policy_grad.reward's per-position rewards, credited per frame as reward-to-go;
-            the baseline is then taken per frame over the K samples)
+            the baseline is then taken per frame over the K samples),
+            'wed' (-word edit distance) or 'wer' (-word edit distance / words in the transcript, as metrics.evaluate's
+            WER): words are split at space_id as str.split(" ") does (empty words kept), which is upstream's string
+            split when every alphabet entry is one character
+    space_id: id of the word separator (alphabet.index(" ")); required by 'wed' / 'wer', must differ from blank
     target_lengths=None: the lengths are taken from the padding -- the number of leading non-zero ids of each row
             (upstream pads transcripts with 0 = '<pad>', data.py:99, which is also the CTC blank and never a label)
     baseline: 'mean' (over the K samples of the utterance), 'loo', 'none', or 'value' (baseline_value)
-    After a call, .last holds rewards [B,K], nll [B], logp [B,K], dist [B,K], hyp_len [B,K].
+    After a call, .last holds rewards [B,K], nll [B], logp [B,K], dist [B,K] (word edit distances for 'wed' / 'wer'),
+    hyp_len [B,K].
     """
 
     def __init__(self, K=16, blank=0, reward="ed", baseline="mean", baseline_value=0.0, pg_weight=1.0,
-                 ctc_weight=1.0, seed=0):
+                 ctc_weight=1.0, seed=0, space_id=None):
         super().__init__()
         if reward not in F.REWARD_MODES or baseline not in F.BASELINE_MODES:
             raise ValueError("unknown reward or baseline mode")
+        if reward in F.WORD_REWARDS:
+            if space_id is None:
+                raise ValueError(f"reward={reward!r} needs space_id, the id of the word separator (alphabet.index(' '))")
+            if int(space_id) == int(blank):
+                raise ValueError("space_id must differ from blank")
+        self.space_id = None if space_id is None else int(space_id)
         self.K, self.blank, self.reward, self.baseline = int(K), int(blank), reward, baseline
         self.baseline_value, self.pg_weight, self.ctc_weight = float(baseline_value), float(pg_weight), float(ctc_weight)
         self.seed, self._calls = int(seed), 0

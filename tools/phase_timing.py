@@ -1,6 +1,8 @@
 """Phase timing of the fused kernel (CTA of utterance 0) from the -DPGASR_TIMING build:
     python policy-gradient-asr_b200/build.py --timing
     PGASR_LIB=policy-gradient-asr_b200/lib/libpgasr_b200_timing.so python tools/phase_timing.py
+PROF_REWARD=wed|wer: the word-level rewards on tools/bench_word_reward.py's text-like transcripts (space id 1;
+PROF_REGIME=random|peaky); the "collapse" phase then includes the word phase, split as W1 (transcripts) / W2.
 """
 import ctypes
 import os
@@ -14,6 +16,12 @@ from tests.synth import make_batch  # noqa: E402
 
 B = int(os.environ.get("PROF_B", "64"))
 dev = torch.device("cuda:0")
+REWARD = os.environ.get("PROF_REWARD", "ed")
+WORD = REWARD in F.WORD_REWARDS
+KW = dict(reward=REWARD, space_id=1) if WORD else {}
+if WORD:
+    from tools.bench_word_reward import text_batch  # noqa: E402
+    make_batch = lambda B_, T_, V_, K_, L_, seed: (*text_batch(seed, os.environ.get("PROF_REGIME", "random")), None)  # noqa: E731
 lg, tg, il, tl, _ = make_batch(B, 500, 30, 16, 100, seed=1)
 t = lambda a: torch.from_numpy(a).to(dev)
 lg, tg, il, tl = t(lg), t(tg), t(il), t(tl)
@@ -22,10 +30,10 @@ buf = (ctypes.c_longlong * 64)()
 ws = None
 for mode, (wp, wc) in {"both": (1.0, 1.0), "ctc": (0.0, 1.0), "pg": (1.0, 0.0)}.items():
     for i in range(3):
-        out = F.pg_ctc_step(lg, tg, il, tl, K=16, seed=i, workspace=ws, pg_weight=wp, ctc_weight=wc)
+        out = F.pg_ctc_step(lg, tg, il, tl, K=16, seed=i, workspace=ws, pg_weight=wp, ctc_weight=wc, **KW)
         ws = out["workspace"]
     lib.pgasr_debug_read(buf, 1)
-    out = F.pg_ctc_step(lg, tg, il, tl, K=16, seed=7, workspace=ws, pg_weight=wp, ctc_weight=wc)
+    out = F.pg_ctc_step(lg, tg, il, tl, K=16, seed=7, workspace=ws, pg_weight=wp, ctc_weight=wc, **KW)
     lib.pgasr_debug_read(buf, 1)
     d = list(buf)
     print(f"== {mode} (cycles)")
@@ -45,10 +53,15 @@ for mode, (wp, wc) in {"both": (1.0, 1.0), "ctc": (0.0, 1.0), "pg": (1.0, 0.0)}.
         names = ["tile-load", "sample", "collapse", "myers", "advantages", "grad-tile", "flag-wait", "rmw-out"]
         print(f" pg sampling split (thread 0): cdf build {d[60]-d[31]}  draws {d[32]-d[60]}")
         print(" pg:  " + "  ".join(f"{n} {d[31+i]-d[30+i]}" for i, n in enumerate(names)) + f"  total {d[38]-d[30]}")
+        if WORD:
+            print(f" pg word phase: collapse {d[61]-d[32]}  W1 transcripts {d[62]-d[61]}  W2 hypotheses {d[33]-d[62]}")
+
+if WORD:       # (the per-CTA wall times below are recorded by the character-mode kernel only)
+    sys.exit(0)
 
 # per-CTA wall times of the last fused launch (globaltimer ns): role start/end spread over the grid
 import numpy as np  # noqa: E402
-out = F.pg_ctc_step(lg, tg, il, tl, K=16, seed=9, workspace=ws)
+out = F.pg_ctc_step(lg, tg, il, tl, K=16, seed=9, workspace=ws, **KW)
 n = 2 * B
 arr = (ctypes.c_ulonglong * (3 * n))()
 assert lib.pgasr_debug_cta_times(arr, n) == 0
@@ -78,7 +91,7 @@ for i in range(8):
     a, b, c, d, _ = make_batch(B, 500, 30, 16, 100, seed=100 + i)
     batches.append({"logits": torch.from_numpy(a).to(dev), "targets": torch.from_numpy(b).to(dev),
                     "in_len": torch.from_numpy(c).to(dev), "tgt_len": torch.from_numpy(d).to(dev)})
-q = F.StepQueue(batches, K=16)
+q = F.StepQueue(batches, K=16, **KW)
 for rep in range(3):
     q.run(first=0, n=8, seed=rep)
 torch.cuda.synchronize()
@@ -94,7 +107,7 @@ for name, sl in (("CTC role CTAs", slice(0, B)), ("PG role CTAs", slice(B, n))):
 if hasattr(lib, "pgasr_debug_role_times"):
     r8 = (ctypes.c_ulonglong * 8)()
     NS = 32                                                # steps per call: fill and drain are ~3 % of a call
-    q = F.StepQueue([batches[i % 8] for i in range(NS)], K=16)
+    q = F.StepQueue([batches[i % 8] for i in range(NS)], K=16, **KW)
     for rep in range(6):
         q.run(first=0, n=NS, seed=10 + rep)
     lib.pgasr_debug_role_times(r8, 1)
