@@ -216,6 +216,21 @@ PGASR_API int pgasr_pg_ctc_step_multi_ws(const pgasr_step_io* steps, int n_steps
                             int reward_mode, int baseline_mode, float baseline_value,
                             float w_pg, float w_ctc, int word_sep,
                             void* workspace, size_t workspace_bytes, void* stream);
+/* The same with the exploration controls (DESIGN.md "exploration spec"): the PG role samples from and trains the
+ * tempered policy softmax(z / temperature), theta = fl32(1 / temperature), and the loss gains an entropy bonus:
+ *   loss = w_pg L_pg + w_ctc mean_b nll_b - w_ent (1/B) sum_b H_b,   H_b = sum_{t < in_len[b]} H(softmax(theta z_bt))
+ * in nats.  The CTC term stays on the untempered logits.  entropy: HOST array of n_steps DEVICE pointers to [B] fp32
+ * that receive H_b (the array or any element may be NULL; an element needs w_pg != 0).  word_sep < 0: no separator
+ * (character modes only); word_sep >= 0: as in pgasr_pg_ctc_step_multi_ws.  Every reward mode is accepted.
+ * PGASR_ERR_INVALID_ARG before any CUDA call: temperature non-finite or outside [0.01, 100], w_ent non-finite or < 0,
+ * w_ent > 0 or an entropy output with w_pg == 0, a bad separator.  With temperature 1, w_ent 0 and no entropy output
+ * the step is exactly the one pgasr_pg_ctc_step_multi (_ws) runs.  Same workspace.                                */
+PGASR_API int pgasr_pg_ctc_step_multi_ex(const pgasr_step_io* steps, int n_steps, uint64_t seed_base,
+                            int B, int T, int V, int K, int Lmax, int blank,
+                            int reward_mode, int baseline_mode, float baseline_value,
+                            float w_pg, float w_ctc, float* const* entropy, int word_sep,
+                            float temperature, float w_ent,
+                            void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- CTC prefix beam search (upstream CTCdecoder.py:41-116, CTCDecoder.decode) -----------------------
  * probs [N,T,V] fp64 post-softmax (upstream takes the post-softmax array and works in Python floats), frames

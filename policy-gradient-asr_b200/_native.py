@@ -34,6 +34,8 @@ SIGNATURES = {
                                _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pgasr_pg_ctc_step_multi": (_i, [_vp, _i, _u64, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _vp, _sz, _vp]),
     "pgasr_pg_ctc_step_multi_ws": (_i, [_vp, _i, _u64, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _i, _vp, _sz, _vp]),
+    "pgasr_pg_ctc_step_multi_ex": (_i, [_vp, _i, _u64, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _vp, _i, _f, _f,
+                                        _vp, _sz, _vp]),
     "pgasr_ctc_beam_search_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "pgasr_ctc_beam_search": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "pgasr_host_create": (_i, [_i, _i, _i, _i, _i, _i, _vp]),

@@ -11,10 +11,14 @@
 namespace pgasr {
 
 constexpr int kFusedMaxK = 64;
-int launch_fused_spl4(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word);
-int launch_fused_spl8(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word);
-int launch_fused_spl16(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word);
-int launch_fused_spl32(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word);
+int launch_fused_spl4(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word,
+                       const ExploreArgs* explore);
+int launch_fused_spl8(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word,
+                       const ExploreArgs* explore);
+int launch_fused_spl16(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word,
+                        const ExploreArgs* explore);
+int launch_fused_spl32(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word,
+                        const ExploreArgs* explore);
 
 constexpr size_t kFusedSmemLimit = 220 * 1024;
 
@@ -144,7 +148,8 @@ size_t fused_workspace_bytes(int B, int T, int V, int K, int Lmax) {
 }
 
 // a.do_pg must be 0 when the PG role does not fit (fused_capability bit 1)
-int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput, const WordArgs* word) {
+int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput, const WordArgs* word,
+               const ExploreArgs* explore) {
     const FusedPlan pl = fused_plan(a.T, a.V, a.K, a.Lmax);
     if (!pl.ctc_ok || (a.do_pg && !pl.pg_ok)) return PGASR_ERR_UNSUPPORTED;
     const FusedWs w = fused_ws(a.B, a.T, a.V, pl.spl, pl.gt);
@@ -180,7 +185,7 @@ int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput, 
     // against 35.78 / 35.66).  Single steps keep it (back-to-back launches on one stream).  PGASR_PDL_THROUGHPUT=1: keep (A/B)
     static const bool pdl_tp = getenv("PGASR_PDL_THROUGHPUT") != nullptr;
     a.no_pdl = throughput && !pdl_tp;
-    if (!a.do_pg) word = nullptr;
+    if (!a.do_pg) word = nullptr, explore = nullptr;
     if (word) {
         // word modes: the same decisions as below on the word layout; the streaming PG role has no word phase
         if (stream || !fused_word_capability(a.T, a.V, a.K, a.Lmax)) return PGASR_ERR_UNSUPPORTED;
@@ -219,10 +224,10 @@ int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput, 
     }
     const int mode = pl.bw ? 3 : !pl.gt ? 0 : !stream ? 1 : 2;   // tiles in shared memory | CTC streams | both stream | block workers
     switch (pl.spl) {
-        case 4: return launch_fused_spl4(mode, a, smem, st, word);
-        case 8: return launch_fused_spl8(mode, a, smem, st, word);
-        case 16: return launch_fused_spl16(mode, a, smem, st, word);
-        default: return launch_fused_spl32(mode, a, smem, st, word);
+        case 4: return launch_fused_spl4(mode, a, smem, st, word, explore);
+        case 8: return launch_fused_spl8(mode, a, smem, st, word, explore);
+        case 16: return launch_fused_spl16(mode, a, smem, st, word, explore);
+        default: return launch_fused_spl32(mode, a, smem, st, word, explore);
     }
 }
 

@@ -30,6 +30,20 @@ struct WordArgs {
     int cap;                 // word_class_cap(Lmax, V): distinct transcript words a hypothesis can match
 };
 
+// Exploration controls (DESIGN.md "exploration spec"): the PG role samples from and trains softmax(theta z), with an
+// entropy bonus.  A kernel argument of its own, like WordArgs, so the default kernels keep their parameter block.
+struct ExploreArgs {
+    float theta;             // fl32(1 / temperature)
+    float ent_c;             // beta / B: the entropy term's gradient is ent_c theta p' (log p' + H_bt)
+    float ent_lt;            // beta K / w_pg: subtracted (times H_b) from the utterance's loss term
+    float* entropy;          // [B] H_b in nats, optional
+};
+
+// Entropy terms of the exploration variant with 0 log 0 = 0: a class whose p' is 0 (underflow, or a logit of -inf, where
+// log p' = -inf) contributes 0 to H and gets gradient 0, instead of 0 * -inf = NaN.
+__device__ __forceinline__ float ent_plogp(float p, float lp) { return p > 0.0f ? p * lp : 0.0f; }
+__device__ __forceinline__ float ent_grad(float p, float c) { return p > 0.0f ? p * c : 0.0f; }
+
 // shared-memory bytes of one utterance's block in a PG CTA (fused_impl.cuh: fused_pg_role; fused.cu sizes with it)
 template <int W, int kThreads>
 __host__ __device__ inline size_t pg_u_bytes(int T, int V, int K) {
@@ -49,11 +63,20 @@ size_t fused_workspace_bytes(int B, int T, int V, int K, int Lmax);
 // throughput: the step is one of several independent ones in flight (pgasr_pg_ctc_step_multi): PG CTAs take two
 // utterances each -- less SM time per step, a longer single step; a step on its own keeps one utterance per PG CTA
 // word (non-NULL): the word-level rewards, a.do_pg set; the PG role must fit in its word layout (fused_word_capability)
-int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput = false, const WordArgs* word = nullptr);
+// explore (non-NULL): the exploration variant of the PG role (a.do_pg set)
+int fused_step(FusedArgs& a, void* workspace, cudaStream_t st, bool throughput = false, const WordArgs* word = nullptr,
+               const ExploreArgs* explore = nullptr);
 // the PG role of the word-level rewards fits an SM (logits tile in shared memory); otherwise the step chains the
 // stand-alone kernels for the PG part
 bool fused_word_capability(int T, int V, int K, int Lmax);
 size_t align256(size_t x);
 void fused_workspace_reset(const void* workspace, size_t bytes);   // forget the control-block parity of every fused workspace in the range
+// chain path of the exploration variant: the sampler on theta z (sampler.cu); the PG gradient with the theta factor,
+// the entropy term and H_b, which it also folds into loss_terms (pg.cu)
+int softmax_sample_theta(const float* logits, const int32_t* in_len, const float* uniforms, uint64_t seed, int B, int T,
+                         int V, int K, float theta, uint8_t* samples, float* logp, float* probs, cudaStream_t st);
+int pg_grad_explore(const float* logits, const uint8_t* samples, const float* adv, const int32_t* in_len, int B, int T,
+                    int V, int K, float scale, bool dense, int accumulate, const ExploreArgs& x, float* loss_terms,
+                    float* dlogits, cudaStream_t st);
 
 }  // namespace pgasr

@@ -411,6 +411,19 @@ __device__ void fused_ctc_role(const FusedArgs& a, int b, unsigned char* smem_ra
     }
 }
 
+// exploration variant: z' = fl32(z theta) over a logits tile in shared memory, float4 where the tile allows
+template <int kThreads>
+__device__ __forceinline__ void scale_tile(float* z, int n, float theta) {
+    float4* z4 = reinterpret_cast<float4*>(z);
+    const int n4 = n / 4;
+    for (int i = threadIdx.x; i < n4; i += kThreads) {
+        float4 x = z4[i];
+        x.x = __fmul_rn(x.x, theta); x.y = __fmul_rn(x.y, theta); x.z = __fmul_rn(x.z, theta); x.w = __fmul_rn(x.w, theta);
+        z4[i] = x;
+    }
+    for (int i = n4 * 4 + threadIdx.x; i < n; i += kThreads) z[i] = __fmul_rn(z[i], theta);
+}
+
 // ------------------------------------------------------------------------------------------------ PG role
 // kStream (long utterances): no [T][V] tile in shared memory -- a thread reads its frame's logits straight from
 // global memory, and the gradient rows are formed in registers and added to dlogits row by row.
@@ -431,13 +444,24 @@ struct PgU {
 // its sequence of word classes, the transcript's words become the match table, and P3 runs over words.
 // (the word arguments come as a parameter pack, empty for the character modes: their role keeps its exact signature --
 // where it is not inlined, an extra parameter changes its call frame)
-__device__ __forceinline__ WordArgs word_args_of() { return WordArgs{-1, 0}; }
-__device__ __forceinline__ WordArgs word_args_of(const WordArgs& w) { return w; }
-template <int W, int kThreads, bool kStream, bool kWord = false, typename... WA>
+// kExp (exploration, DESIGN.md "exploration spec"): the logits are scaled by theta -- the tile once after its load, the
+// streamed rows on read -- so P1 samples softmax(theta z); P5 multiplies the coefficients by theta and adds the
+// entropy term, and writes H_b.  Its ExploreArgs come last in the same pack.
+struct PgExtra { WordArgs w; ExploreArgs x; };
+__device__ __forceinline__ PgExtra pg_extra() { return PgExtra{{-1, 0}, {1.0f, 0.0f, 0.0f, nullptr}}; }
+__device__ __forceinline__ PgExtra pg_extra(const WordArgs& w) { return PgExtra{w, {1.0f, 0.0f, 0.0f, nullptr}}; }
+__device__ __forceinline__ PgExtra pg_extra(const ExploreArgs& x) { return PgExtra{{-1, 0}, x}; }
+__device__ __forceinline__ PgExtra pg_extra(const WordArgs& w, const ExploreArgs& x) { return PgExtra{w, x}; }
+template <int W, int kThreads, bool kStream, bool kWord = false, bool kExp = false, typename... XA>
 __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned char* smem_raw, unsigned* s_last,
-                              unsigned long long* s_mbar, const WA&... word) {
-    static_assert(kWord == (sizeof...(WA) == 1), "the word modes take their WordArgs, the character modes none");
-    const WordArgs wa = word_args_of(word...);
+                              unsigned long long* s_mbar, const XA&... extra) {
+    static_assert(sizeof...(XA) == (kWord ? 1 : 0) + (kExp ? 1 : 0), "WordArgs for the word modes, then ExploreArgs");
+    const PgExtra px = pg_extra(extra...);
+    const WordArgs wa = px.w;
+    const float theta = px.x.theta;
+    (void)theta;
+    // a value of the frame's row as the policy sees it: streamed rows are scaled on read, the tile already is
+    auto zv = [&](const float* z, int v) { return kExp && kStream ? __fmul_rn(z[v], theta) : z[v]; };
     constexpr int kWarps = kThreads / 32;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int T = a.T, V = a.V, K = a.K;
@@ -529,6 +553,12 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
         if (!kStream && a.bulk_tile) mbar_wait(s_mbar, nload++ & 1u);
         cp_async_wait<0>();
         __syncthreads();
+        if constexpr (kExp && !kStream) {
+            if (theta != 1.0f) {                           // z' = z theta, once per tile (theta = 1: z' = z bit for bit)
+                scale_tile<kThreads>(ztile, T * V, theta);
+                __syncthreads();
+            }
+        }
 
 
         PGASR_STAMP(dbg, 31);
@@ -545,7 +575,7 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
                 float mx = -INFINITY, S = 0.0f, logS = 0.0f;
                 if (live) {
 #pragma unroll
-                    for (int v = 0; v < VPW; ++v) cdf[v] = v < V ? z[v] : -INFINITY;
+                    for (int v = 0; v < VPW; ++v) cdf[v] = v < V ? zv(z, v) : -INFINITY;
 #pragma unroll
                     for (int v = 0; v < VPW; ++v) mx = fmaxf(mx, cdf[v]);
                     float c = 0.0f;
@@ -586,7 +616,7 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
                             cnt = (hi ? 32 : 0) + cdf_count32(half, tau);
                         }
                         pi = min(cnt, V - 1);
-                        term = (z[pi] - mx) - logS;
+                        term = (zv(z, pi) - mx) - logS;
                     }
                     if (t < T) {
                         samples_s[(size_t)k * Tp + t] = (uint8_t)pi;
@@ -1103,20 +1133,62 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
         (void)dbg; (void)samples_s; (void)hyp_s; (void)hrev_s; (void)peq; (void)peq_r; (void)fg_s; (void)warp_acc; (void)adv_s;
         (void)hlen_s; (void)dist_s; (void)misc_s; (void)lg; (void)ref; (void)Tb; (void)m;
         PGASR_STAMP(dbg, 35);
+        const bool dense = a.baseline_mode != PGASR_BASELINE_MEAN;   // sum_k A_k == 0 under the per-utterance mean
+        // exploration: the entropy term (or its output) needs the dense softmax under every baseline
+        const bool ent = kExp && (px.x.ent_c != 0.0f || px.x.entropy != nullptr);
         if (!kStream && uu != nutt - 1) {
-            if (a.baseline_mode != PGASR_BASELINE_MEAN) { // (the tile holds the previous utterance's gradient)
+            if (dense || ent) {                            // (the tile holds the previous utterance's gradient)
                 if (a.bulk_tile) {
                     if (threadIdx.x == 0) bulk_load_tile(ztile, lg, (unsigned)((size_t)T * V * 4), s_mbar);
                     mbar_wait(s_mbar, nload++ & 1u);
                 } else {
                     for (int i = threadIdx.x; i < T * V; i += kThreads) ztile[i] = __ldg(lg + i);
                 }
+                if constexpr (kExp) {
+                    if (theta != 1.0f) {
+                        __syncthreads();
+                        scale_tile<kThreads>(ztile, T * V, theta);
+                    }
+                }
             }
             __syncthreads();
         }
         // ---- P5: REINFORCE gradient tile, in place of the logits tile ---------------------------------
-        const float coef = a.w_pg / ((float)a.B * (float)K);
-        const bool dense = a.baseline_mode != PGASR_BASELINE_MEAN;   // sum_k A_k == 0 under the per-utterance mean
+        // (exploration: times theta, the chain factor of z' = theta z)
+        const float coef = kExp ? __fmul_rn(a.w_pg / ((float)a.B * (float)K), theta) : a.w_pg / ((float)a.B * (float)K);
+        const float ent_c = kExp ? __fmul_rn(px.x.ent_c, theta) : 0.0f;
+        double hsum = 0.0;                                     // exploration: this thread's frames' H_bt
+        (void)ent_c; (void)hsum;
+        // exploration: the gradient row of a frame from its z' row (in place): theta (coef sum_k A_k p' [dense] +
+        // (beta / B) p' (log p' + H_t)) -- the sample terms follow; returns H_t
+        auto explore_row = [&](float* row, float lz, float dcoef) {
+            float H = 0.0f;
+            for (int v = 0; v < V; ++v) {
+                const float lp = row[v] - lz;                  // log p' = z' - m' - ln S, never log(p')
+                H -= ent_plogp(__expf(lp), lp);
+            }
+            for (int v = 0; v < V; ++v) {
+                const float lp = row[v] - lz, p = __expf(lp);
+                row[v] = ent_grad(p, dcoef + (ent ? ent_c * (lp + H) : 0.0f));
+            }
+            return H;
+        };
+        (void)explore_row;
+        // exploration: H_b = sum of the frames' H_t in a fixed order (threads -> warps -> warp 0..), the entropy output,
+        // and - beta K / w_pg H_b folded into the utterance's loss term (the loss then carries -beta / B sum_b H_b).  The
+        // loss term must be final before this CTA draws its done ticket.
+        auto explore_finish = [&]() {
+            hsum = warp_sum(hsum);
+            if (lane == 0) warp_acc[32 + warp] = hsum;     // (P4 has consumed the log-prob partial sums)
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                double H = 0.0;
+                for (int w = 0; w < kWarps; ++w) H += warp_acc[32 + w];
+                if (px.x.entropy) px.x.entropy[b] = (float)H;
+                if (px.x.ent_lt != 0.0f) a.loss_terms[b] = (float)((double)a.loss_terms[b] - (double)px.x.ent_lt * H);
+            }
+        };
+        (void)explore_finish;
         const float dense_c = coef * misc_s[0];
         float* dlog_u = a.dlogits + (size_t)b * T * V;
         const bool final_u = uu == 0;                          // the last utterance this CTA finishes: it draws the done ticket
@@ -1128,7 +1200,7 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
                     const unsigned* flag = a.ctrl + 4 + b;
                     while (ld_acquire(flag) == 0u) __nanosleep(40);
                 }
-                if (final_u) draw_done_ticket(a, s_last);
+                if (final_u && !ent) draw_done_ticket(a, s_last);
             }
             __syncthreads();
             PGASR_STAMP(dbg, 37);
@@ -1139,20 +1211,40 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
                         for (int v = 0; v < V; ++v) out[v] = 0.0f;
                     continue;
                 }
-                float mx = 0.0f, sc = 0.0f;
+                float mx = 0.0f, sc = 0.0f, lz = 0.0f, H = 0.0f;
                 const float* zr = lg + (size_t)t * V;
-                if (dense) {
+                if (dense || ent) {
                     mx = -INFINITY;
                     float ssum = 0.0f;
-                    for (int v = 0; v < V; ++v) mx = fmaxf(mx, zr[v]);
-                    for (int v = 0; v < V; ++v) ssum += __expf(zr[v] - mx);
+                    for (int v = 0; v < V; ++v) mx = fmaxf(mx, zv(zr, v));
+                    for (int v = 0; v < V; ++v) ssum += __expf(zv(zr, v) - mx);
                     sc = dense_c / ssum;
+                    if (ent) {                                 // H_t = -sum_v p' log p', log p' = z' - m' - ln S
+                        lz = mx + logf(ssum);
+                        for (int v = 0; v < V; ++v) {
+                            const float lp = zv(zr, v) - lz;
+                            H -= ent_plogp(__expf(lp), lp);
+                        }
+                        hsum += (double)H;
+                    }
                 }
                 for (int v = 0; v < V; ++v) {
-                    float g = dense ? __expf(zr[v] - mx) * sc : 0.0f;
+                    float g;
+                    if (ent) {
+                        const float lp = zv(zr, v) - lz;
+                        g = ent_grad(__expf(lp), (dense ? dense_c : 0.0f) + ent_c * (lp + H));
+                    } else {
+                        g = dense ? __expf(zv(zr, v) - mx) * sc : 0.0f;
+                    }
                     for (int k = 0; k < K; ++k)              // same order of subtractions as the tile mode: k ascending
                         if (samples_s[(size_t)k * Tp + t] == v) g -= coef * adv_s[k];
                     out[v] = a.do_ctc ? __ldcg(out + v) + g : g;
+                }
+            }
+            if constexpr (kExp) {
+                if (ent) {                                     // (the ticket after the loss term is final)
+                    explore_finish();
+                    if (threadIdx.x == 0 && final_u) draw_done_ticket(a, s_last);
                 }
             }
             PGASR_STAMP(dbg, 38);
@@ -1182,7 +1274,9 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
                         lt += -(double)A * (double)(row[samples_s[(size_t)k * Tp + t]] - lz);
                         sumA += A;
                     }
-                    if (dense) {
+                    if (ent) {
+                        hsum += (double)explore_row(row, lz, dense ? coef * sumA : 0.0f);
+                    } else if (dense) {
                         const float sc = coef * sumA;
                         for (int v = 0; v < V; ++v) row[v] = __expf(row[v] - lz) * sc;
                     } else {
@@ -1206,7 +1300,12 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
         for (int t = threadIdx.x; t < T; t += kThreads) {
             float* row = ztile + (size_t)t * V;
             if (t < Tb) {
-                if (dense) {
+                if (ent) {
+                    float mx = -INFINITY, s = 0.0f;
+                    for (int v = 0; v < V; ++v) mx = fmaxf(mx, row[v]);
+                    for (int v = 0; v < V; ++v) s += __expf(row[v] - mx);
+                    hsum += (double)explore_row(row, mx + logf(s), dense ? dense_c : 0.0f);
+                } else if (dense) {
                     float mx = -INFINITY, s = 0.0f;
                     for (int v = 0; v < V; ++v) mx = fmaxf(mx, row[v]);
                     for (int v = 0; v < V; ++v) s += __expf(row[v] - mx);
@@ -1221,6 +1320,9 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
             }
         }
         __syncthreads();
+        if constexpr (kExp) {
+            if (ent) explore_finish();                     // (thread 0 draws the done ticket below, after this)
+        }
 
         PGASR_STAMP(dbg, 36);
         // ---- P6: add the tile onto the CTC rows (or store it when there is no CTC term) ---------------
@@ -1368,6 +1470,39 @@ __global__ void __launch_bounds__(kThreads, 1) pg_ctc_fused_word_kernel(const Fu
     if (s_last && threadIdx.x < 32 && ticket < n_ctc) loss_reduce_and_rearm(a);
 }
 
+// exploration (temperature / entropy bonus, character or word modes): the kernels above with the exploration variant of
+// the PG role (fused_pg_role<..., kExp = true>); same ticket protocol, no timing stamps
+template <int SPL, int kThreads, bool kGT, bool kStream, bool kBW, bool kWord>
+__global__ void __launch_bounds__(kThreads, 1) pg_ctc_fused_explore_kernel(const FusedArgs a, const WordArgs wa,
+                                                                           const ExploreArgs x) {
+    static_assert(!(kWord && kStream), "the streaming PG role has no word phase");
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ unsigned s_ticket, s_last;
+    __shared__ __align__(8) unsigned long long s_mbar;
+    if (threadIdx.x == 0 && a.bulk_tile) {
+        mbar_init(&s_mbar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    }
+    if (threadIdx.x == 0) s_ticket = atomicAdd(a.ctrl, 1u);
+    __syncthreads();
+    asm volatile("griddepcontrol.wait;\n" ::: "memory");
+    asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory");
+    const unsigned ticket = s_ticket;
+    const unsigned n_ctc = a.do_ctc ? (unsigned)a.B : 0u;
+    if (ticket < n_ctc) fused_ctc_role<SPL, kThreads, kGT, kBW>(a, (int)ticket, smem_raw, &s_last, &s_mbar);
+    else {
+        const int j = (int)(ticket - n_ctc);
+        const int b0 = a.pg_pair ? 2 * j : j;
+        const int nutt = a.pg_pair ? min(2, a.B - b0) : 1;
+        if constexpr (kWord)
+            fused_pg_role<SPL / 2, kThreads, false, true, true>(a, b0, nutt, smem_raw, &s_last, &s_mbar, wa, x);
+        else
+            fused_pg_role<SPL / 2, kThreads, kStream, false, true>(a, b0, nutt, smem_raw, &s_last, &s_mbar, x);
+    }
+    __syncthreads();
+    if (s_last && threadIdx.x < 32 && (ticket < n_ctc || kStream)) loss_reduce_and_rearm(a);
+}
+
 // the dynamic shared-memory opt-in of `kern`: sticky PER DEVICE, raised only when a larger tile comes on the device the
 // launch goes to (smem_set: one per kernel)
 template <typename Kern>
@@ -1381,17 +1516,31 @@ static int fused_smem_optin(Kern kern, size_t (&smem_set)[64], size_t smem) {
     return PGASR_OK;
 }
 
+template <int SPL, int kThreads, bool kGT, bool kStream, bool kBW, bool kWord>
+static int launch_fused_explore(FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word, const ExploreArgs& x,
+                                cudaLaunchConfig_t& cfg) {
+    static thread_local size_t smem_set[64] = {0};
+    const auto kern = pg_ctc_fused_explore_kernel<SPL, kThreads, kGT, kStream, kBW, kWord>;
+    const int rc = fused_smem_optin(kern, smem_set, smem);
+    if (rc) return rc;
+    const WordArgs wa = word ? *word : WordArgs{-1, 0};
+    PGASR_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, a, wa, x));
+    ++g_launches;
+    return PGASR_OK;
+}
+
 template <int SPL, int kThreads, bool kGT, bool kStream, bool kBW = false>
-static int launch_fused(FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word = nullptr) {
+static int launch_fused(FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word = nullptr,
+                        const ExploreArgs* explore = nullptr) {
     static thread_local size_t smem_set[64] = {0};
     static thread_local size_t smem_set_w[64] = {0};
     if constexpr (!kStream) {
-        if (word) {
+        if (word && !explore) {
             const int rc = fused_smem_optin(pg_ctc_fused_word_kernel<SPL, kThreads, kGT, kBW>, smem_set_w, smem);
             if (rc) return rc;
         }
     }
-    if (!word) {
+    if (!word && !explore) {
         const int rc = fused_smem_optin(pg_ctc_fused_kernel<SPL, kThreads, kGT, kStream, kBW>, smem_set, smem);
         if (rc) return rc;
     }
@@ -1407,6 +1556,13 @@ static int launch_fused(FusedArgs& a, size_t smem, cudaStream_t st, const WordAr
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = (no_pdl || a.no_pdl) ? 0 : 1;
+    if (explore) {
+        if constexpr (!kStream) {
+            if (word) return launch_fused_explore<SPL, kThreads, kGT, kStream, kBW, true>(a, smem, st, word, *explore, cfg);
+        }
+        if (word) return PGASR_ERR_UNSUPPORTED;
+        return launch_fused_explore<SPL, kThreads, kGT, kStream, kBW, false>(a, smem, st, word, *explore, cfg);
+    }
     if constexpr (!kStream) {
         if (word) {
             PGASR_CUDA_TRY(cudaLaunchKernelEx(&cfg, pg_ctc_fused_word_kernel<SPL, kThreads, kGT, kBW>, a, *word));
@@ -1424,15 +1580,17 @@ static int launch_fused(FusedArgs& a, size_t smem, cudaStream_t st, const WordAr
 // 2: both roles stream, 3: tiles in shared memory with block workers -- up to 8 states per lane only) so that the
 // variants compile in parallel
 // word (non-NULL): the word-mode kernel, modes 0, 1 and 3 (the PG role keeps its tile in shared memory)
+// explore (non-NULL): the exploration variant of either
 template <int SPL, int kThreads>
-int launch_fused_modes(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word) {
+int launch_fused_modes(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word,
+                       const ExploreArgs* explore) {
     if constexpr (SPL <= 8) {
-        if (mode == 3) return launch_fused<SPL, kThreads, false, false, true>(a, smem, st, word);
+        if (mode == 3) return launch_fused<SPL, kThreads, false, false, true>(a, smem, st, word, explore);
     }
     switch (mode) {
-        case 0: return launch_fused<SPL, kThreads, false, false>(a, smem, st, word);
-        case 1: return launch_fused<SPL, kThreads, true, false>(a, smem, st, word);
-        default: return launch_fused<SPL, kThreads, true, true>(a, smem, st, word);
+        case 0: return launch_fused<SPL, kThreads, false, false>(a, smem, st, word, explore);
+        case 1: return launch_fused<SPL, kThreads, true, false>(a, smem, st, word, explore);
+        default: return launch_fused<SPL, kThreads, true, true>(a, smem, st, word, explore);
     }
 }
 

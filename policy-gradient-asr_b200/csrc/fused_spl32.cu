@@ -2,7 +2,8 @@
 #include "fused_impl.cuh"
 
 namespace pgasr {
-int launch_fused_spl32(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word) {
-    return launch_fused_modes<32, 256>(mode, a, smem, st, word);
+int launch_fused_spl32(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word,
+                      const ExploreArgs* explore) {
+    return launch_fused_modes<32, 256>(mode, a, smem, st, word, explore);
 }
 }  // namespace pgasr

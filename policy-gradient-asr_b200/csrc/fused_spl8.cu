@@ -2,8 +2,9 @@
 #include "fused_impl.cuh"
 
 namespace pgasr {
-int launch_fused_spl8(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word) {
-    return launch_fused_modes<8, 512>(mode, a, smem, st, word);
+int launch_fused_spl8(int mode, FusedArgs& a, size_t smem, cudaStream_t st, const WordArgs* word,
+                      const ExploreArgs* explore) {
+    return launch_fused_modes<8, 512>(mode, a, smem, st, word, explore);
 }
 }  // namespace pgasr
 

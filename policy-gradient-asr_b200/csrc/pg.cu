@@ -1,7 +1,7 @@
 // K4: rewards, baseline, advantages and the REINFORCE gradient scatter (SURVEY.md 8a row a7; no upstream
 // code -- the reward follows metrics.py:24-25 (ED, or ED / len(reference))), and the customNLLLoss slot
 // (row a5, upstream loss.py:13-17).
-#include "pgasr_common.cuh"
+#include "fused_args.cuh"
 
 namespace pgasr {
 
@@ -65,6 +65,78 @@ __global__ void pg_grad_kernel(const uint8_t* __restrict__ samples, const float*
         g *= scale;
     }
     dlogits[idx] = accumulate ? dlogits[idx] + g : g;
+}
+
+// Exploration variant (DESIGN.md "exploration spec"), one CTA per utterance, one thread per frame: the frame's row of
+// p' = softmax(theta z) from the logits, then dlogits[b,t,v] (+)= theta (scale (p' sum_k A_k [dense] - sum_k A_k
+// [pi_kt = v]) + (beta / B) p' (log p' + H_t)); H_b = sum_t H_t in a fixed order goes to the entropy output and, times
+// beta K / w_pg, out of the utterance's loss term (written by pg_advantages_kernel before this kernel runs).
+constexpr int kPgxThreads = 256;
+__global__ void __launch_bounds__(kPgxThreads)
+pg_grad_explore_kernel(const float* __restrict__ logits, const uint8_t* __restrict__ samples,
+                       const float* __restrict__ adv, const int32_t* __restrict__ in_len, int T, int V, int K,
+                       float scale, int dense, int accumulate, const ExploreArgs x, float* __restrict__ loss_terms,
+                       float* __restrict__ dlogits) {
+    __shared__ double ent_w[kPgxThreads / kWarp];
+    const int b = blockIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int Tb = in_len ? min(max(in_len[b], 0), T) : T;
+    const float* A = adv + (size_t)b * K;
+    float sumA = 0.0f;
+    for (int k = 0; k < K; ++k) sumA += __ldg(A + k);
+    const bool ent = x.ent_c != 0.0f || x.entropy != nullptr;
+    const float th = x.theta, c = __fmul_rn(scale, th), ec = __fmul_rn(x.ent_c, th);
+    double hsum = 0.0;
+    for (int t = threadIdx.x; t < T; t += kPgxThreads) {
+        float* out = dlogits + ((size_t)b * T + t) * V;
+        if (t >= Tb) {
+            if (!accumulate)
+                for (int v = 0; v < V; ++v) out[v] = 0.0f;
+            continue;
+        }
+        const float* z = logits + ((size_t)b * T + t) * V;
+        float m = -INFINITY, S = 0.0f;
+        for (int v = 0; v < V; ++v) m = fmaxf(m, __fmul_rn(__ldg(z + v), th));
+        for (int v = 0; v < V; ++v) S += __expf(__fmul_rn(__ldg(z + v), th) - m);
+        const float lz = m + logf(S);
+        float H = 0.0f;
+        if (ent) {
+            for (int v = 0; v < V; ++v) {
+                const float lp = __fmul_rn(__ldg(z + v), th) - lz;      // log p' = z' - m' - ln S, never log(p')
+                H -= ent_plogp(__expf(lp), lp);
+            }
+            hsum += (double)H;
+        }
+        for (int v = 0; v < V; ++v) {
+            const float lp = __fmul_rn(__ldg(z + v), th) - lz, p = __expf(lp);
+            float hit = 0.0f;
+            for (int k = 0; k < K; ++k)
+                if (samples[((size_t)b * K + k) * T + t] == v) hit += __ldg(A + k);
+            float g = c * ((dense ? p * sumA : 0.0f) - hit);
+            if (ent) g += ent_grad(p, ec * (lp + H));
+            out[v] = accumulate ? out[v] + g : g;
+        }
+    }
+    hsum = warp_sum(hsum);
+    if (lane == 0) ent_w[warp] = hsum;
+    __syncthreads();
+    if (threadIdx.x == 0 && ent) {
+        double Hb = 0.0;
+        for (int w = 0; w < kPgxThreads / kWarp; ++w) Hb += ent_w[w];
+        if (x.entropy) x.entropy[b] = (float)Hb;
+        if (x.ent_lt != 0.0f && loss_terms) loss_terms[b] = (float)((double)loss_terms[b] - (double)x.ent_lt * Hb);
+    }
+}
+
+int pg_grad_explore(const float* logits, const uint8_t* samples, const float* adv, const int32_t* in_len, int B, int T,
+                    int V, int K, float scale, bool dense, int accumulate, const ExploreArgs& x, float* loss_terms,
+                    float* dlogits, cudaStream_t st) {
+    if (!logits || !samples || !adv || !dlogits || B < 0 || T <= 0 || V <= 0 || K <= 0) return PGASR_ERR_INVALID_ARG;
+    if (B == 0) return PGASR_OK;
+    pg_grad_explore_kernel<<<B, kPgxThreads, 0, st>>>(logits, samples, adv, in_len, T, V, K, scale, dense ? 1 : 0,
+                                                      accumulate, x, loss_terms, dlogits);
+    PGASR_LAUNCH_CHECK();
+    return PGASR_OK;
 }
 
 // customNLLLoss.forward (loss.py:13-17): one CTA, deterministic order.  step i: mean over the

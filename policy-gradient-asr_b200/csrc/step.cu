@@ -1,5 +1,6 @@
 // The whole loss step behind one C-ABI call (upstream call site: criterion(model_out, t) followed by
 // loss.backward(), model.py:235-237), plus the small ABI utilities.
+#include <cmath>
 #include <cstdlib>
 
 #include "fused_args.cuh"
@@ -151,6 +152,7 @@ struct StepParams {
     int B, T, V, K, Lmax, blank, reward_mode, baseline_mode;
     float baseline_value, w_pg, w_ctc;
     int word_sep;            // -1: entry points without word modes (reward_mode <= PGASR_REWARD_MAX)
+    float temperature = 1.0f, w_ent = 0.0f;   // exploration (pgasr_pg_ctc_step_multi_ex)
 };
 
 static bool word_mode(int reward_mode) {
@@ -174,8 +176,9 @@ static int step_check(const StepParams& q, const void* workspace, size_t workspa
 }
 
 // one step: one launch of the single-launch kernel when the shape fits, else the chain of stand-alone kernels
+// entropy: the step's H_b output (pgasr_pg_ctc_step_multi_ex), or NULL
 static int step_one(const StepParams& q, const pgasr_step_io& io, uint64_t seed, void* workspace, cudaStream_t st,
-                    bool throughput = false) {
+                    bool throughput = false, float* entropy = nullptr) {
     if (!io.logits || !io.targets || !io.loss || !io.dlogits) return PGASR_ERR_INVALID_ARG;
     void* stream = reinterpret_cast<void*>(st);
     const int B = q.B, T = q.T, V = q.V, K = q.K, Lmax = q.Lmax;
@@ -185,6 +188,13 @@ static int step_one(const StepParams& q, const pgasr_step_io& io, uint64_t seed,
     // word modes: the single-launch kernel when its word layout fits, else the PG part chains the stand-alone kernels
     const bool words_fused = words && do_pg && fused_word_capability(T, V, K, Lmax);
     const WordArgs wa = {q.word_sep, word_class_cap(Lmax, V)};
+    // exploration variant only when it changes something: defaults launch the kernels they always launched
+    const bool explore = do_pg && (q.temperature != 1.0f || q.w_ent != 0.0f || entropy);
+    ExploreArgs x;
+    x.theta = 1.0f / q.temperature;                        // theta = fl32(1 / tau)
+    x.ent_c = q.w_ent / (float)B;
+    x.ent_lt = q.w_ent != 0.0f ? q.w_ent * (float)K / q.w_pg : 0.0f;
+    x.entropy = entropy;
     FusedArgs a;
     a.logits = io.logits; a.targets = io.targets; a.in_len = io.in_len; a.tgt_len = io.tgt_len; a.uniforms = io.uniforms;
     a.seed = seed; a.B = B; a.T = T; a.V = V; a.K = K; a.Lmax = Lmax; a.blank = q.blank;
@@ -194,7 +204,7 @@ static int step_one(const StepParams& q, const pgasr_step_io& io, uint64_t seed,
     a.dist = io.dist; a.nll = io.nll; a.samples = io.samples; a.to_go = io.to_go; a.r_pos = io.r_pos;
     if ((do_pg || do_ctc) && (cap & 1) && (!do_pg || (cap & 2)) && (!words || !do_pg || words_fused)) {
         // one launch: heterogeneous CTAs (CTC role / PG role per utterance), see fused.cu
-        return fused_step(a, workspace, st, throughput, words && do_pg ? &wa : nullptr);
+        return fused_step(a, workspace, st, throughput, words && do_pg ? &wa : nullptr, explore ? &x : nullptr);
     }
     if (do_pg && q.reward_mode == PGASR_REWARD_ED_TO_GO) return PGASR_ERR_UNSUPPORTED;   // (single-launch kernel only)
     // long utterances: the PG role's tiles do not fit one SM -- the PG part runs as the chain of stand-alone
@@ -211,8 +221,10 @@ static int step_one(const StepParams& q, const pgasr_step_io& io, uint64_t seed,
     const bool dense = q.baseline_mode != PGASR_BASELINE_MEAN;   // sum_k A_k == 0 under the per-utterance mean
     int rc;
     if (do_pg || do_ctc) {
-        // the sampler also produces the softmax the CTC lattice and the dense PG term read
-        rc = pgasr_softmax_sample(io.logits, io.in_len, io.uniforms, seed, B, T, V, K, smp, lp, w.probs, stream);
+        // the sampler also produces the softmax the CTC lattice and the dense PG term read (exploration: it samples
+        // softmax(theta z); the gradient kernel then forms p' itself and the CTC kernel its softmax of z)
+        rc = explore ? softmax_sample_theta(io.logits, io.in_len, io.uniforms, seed, B, T, V, K, x.theta, smp, lp, nullptr, st)
+                     : pgasr_softmax_sample(io.logits, io.in_len, io.uniforms, seed, B, T, V, K, smp, lp, w.probs, stream);
         if (rc) return rc;
     }
     if (do_pg) {
@@ -243,11 +255,15 @@ static int step_one(const StepParams& q, const pgasr_step_io& io, uint64_t seed,
         rc = fused_step(a, workspace, st);                 // dlogits = (w_ctc / B) g_ctc, nll; loss is finalised below
         if (rc) return rc;
     } else if (do_ctc) {
-        rc = pgasr_ctc_loss_grad(io.logits, w.probs, io.targets, io.in_len, io.tgt_len, B, T, V, Lmax, q.blank,
+        rc = pgasr_ctc_loss_grad(io.logits, explore ? nullptr : w.probs, io.targets, io.in_len, io.tgt_len, B, T, V, Lmax, q.blank,
                                  q.w_ctc / (float)B, 0, nl, io.dlogits, w.ctc, w.ctc_bytes, stream);
         if (rc) return rc;
     }
-    if (do_pg) {
+    if (do_pg && explore) {
+        rc = pg_grad_explore(io.logits, smp, w.adv, io.in_len, B, T, V, K, q.w_pg / ((float)B * (float)K), dense,
+                             do_ctc ? 1 : 0, x, w.loss_terms, io.dlogits, st);
+        if (rc) return rc;
+    } else if (do_pg) {
         rc = pgasr_pg_grad(smp, w.adv, dense ? w.probs : nullptr, io.in_len, B, T, V, K,
                            q.w_pg / ((float)B * (float)K), do_ctc ? 1 : 0, io.dlogits, stream);
         if (rc) return rc;
@@ -312,7 +328,7 @@ static int aux_lane(AuxLane** out) {
 // events, so to the caller the call is ordered on `stream` like any other.  PGASR_NO_OVERLAP=1: one stream.
 namespace pgasr {
 static int step_multi(const StepParams& q, const pgasr_step_io* steps, int n_steps, uint64_t seed_base,
-                      void* workspace, size_t workspace_bytes, void* stream);
+                      void* workspace, size_t workspace_bytes, void* stream, float* const* entropy = nullptr);
 }
 
 extern "C" int pgasr_pg_ctc_step_multi(const pgasr_step_io* steps, int n_steps, uint64_t seed_base, int B, int T,
@@ -335,9 +351,30 @@ extern "C" int pgasr_pg_ctc_step_multi_ws(const pgasr_step_io* steps, int n_step
     return step_multi(q, steps, n_steps, seed_base, workspace, workspace_bytes, stream);
 }
 
+// the same with the exploration controls and every reward mode (word_sep < 0: no separator, character modes only)
+extern "C" int pgasr_pg_ctc_step_multi_ex(const pgasr_step_io* steps, int n_steps, uint64_t seed_base, int B, int T,
+                                          int V, int K, int Lmax, int blank, int reward_mode, int baseline_mode,
+                                          float baseline_value, float w_pg, float w_ctc, float* const* entropy,
+                                          int word_sep, float temperature, float w_ent, void* workspace,
+                                          size_t workspace_bytes, void* stream) {
+    using namespace pgasr;
+    if (!std::isfinite(temperature) || !(temperature >= 0.01f && temperature <= 100.0f)) return PGASR_ERR_INVALID_ARG;
+    if (!std::isfinite(w_ent) || !(w_ent >= 0.0f) || (w_ent > 0.0f && w_pg == 0.0f)) return PGASR_ERR_INVALID_ARG;
+    if (word_sep >= 0 && (word_sep >= V || word_sep == blank)) return PGASR_ERR_INVALID_ARG;
+    if (!steps || n_steps < 0) return PGASR_ERR_INVALID_ARG;
+    if (entropy && w_pg == 0.0f)                           // (H_b comes from the PG role)
+        for (int i = 0; i < n_steps; ++i)
+            if (entropy[i]) return PGASR_ERR_INVALID_ARG;
+    StepParams q = {B, T, V, K, Lmax, blank, reward_mode, baseline_mode, baseline_value, w_pg, w_ctc,
+                    word_sep < 0 ? -1 : word_sep};
+    q.temperature = temperature;
+    q.w_ent = w_ent;
+    return step_multi(q, steps, n_steps, seed_base, workspace, workspace_bytes, stream, entropy);
+}
+
 namespace pgasr {
 static int step_multi(const StepParams& q, const pgasr_step_io* steps, int n_steps, uint64_t seed_base,
-                      void* workspace, size_t workspace_bytes, void* stream) {
+                      void* workspace, size_t workspace_bytes, void* stream, float* const* entropy) {
     const int B = q.B, T = q.T, V = q.V, K = q.K, Lmax = q.Lmax;
     if (!steps || n_steps < 0) return PGASR_ERR_INVALID_ARG;
     int rc = step_check(q, workspace, workspace_bytes);
@@ -356,7 +393,7 @@ static int step_multi(const StepParams& q, const pgasr_step_io* steps, int n_ste
     for (int i = 0; i < n_steps; ++i) {
         const int l = i % nl;
         rc = step_one(q, steps[i], seed_base + steps[i].seed, reinterpret_cast<char*>(workspace) + (size_t)l * lane_bytes,
-                      l ? aux->stream[l - 1] : s0, nl > 1);
+                      l ? aux->stream[l - 1] : s0, nl > 1, entropy ? entropy[i] : nullptr);
         if (rc) break;
     }
     for (int l = 1; l < nl; ++l) {                         // join, also after an error: the caller's stream stays the one order

@@ -5,6 +5,7 @@ stream through the C ABI (include/pgasr.h) and returns CUDA tensors.  torch is u
 and streams only.  There is no CPU path: a CPU tensor is a TypeError, a missing library a RuntimeError.
 """
 import ctypes as C
+import math
 
 import torch
 
@@ -14,6 +15,7 @@ REWARD_MODES = {"ed": 0, "cer": 1, "ed_to_go": 2, "wed": 3, "wer": 4}
 WORD_REWARDS = ("wed", "wer")      # word-level: need the separator id (space_id), pgasr_pg_ctc_step_multi_ws
 NO_IGNORE = -2**31                  # PGASR_NO_IGNORE
 OPTIONAL_OUTPUTS = ("rewards", "logp", "hyp_len", "dist", "nll", "samples", "to_go", "r_pos")
+EXPLORE_OUTPUTS = ("entropy",)      # H_b [B]: pgasr_pg_ctc_step_multi_ex only (not a field of pgasr_step_io)
 BASELINE_MODES = {"none": 0, "mean": 1, "loo": 2, "value": 3}
 
 
@@ -290,7 +292,8 @@ class StepWorkspace:
 
 
 _OUT_DTYPES = {"rewards": torch.float32, "logp": torch.float32, "hyp_len": torch.int32, "dist": torch.int32,
-               "nll": torch.float32, "samples": torch.uint8, "to_go": torch.int16, "r_pos": torch.int8}
+               "nll": torch.float32, "samples": torch.uint8, "to_go": torch.int16, "r_pos": torch.int8,
+               "entropy": torch.float32}
 
 
 def _alloc_outputs(key, dev, want):
@@ -298,9 +301,9 @@ def _alloc_outputs(key, dev, want):
     out = {"loss": torch.empty((1,), dtype=torch.float32, device=dev),
            "dlogits": torch.empty((B, T, V), dtype=torch.float32, device=dev)}
     for name in want:
-        if name not in OPTIONAL_OUTPUTS:
-            raise ValueError(f"unknown output {name!r}; choose from {OPTIONAL_OUTPUTS}")
-        shape = (B,) if name == "nll" else (B, K, T) if name in ("samples", "to_go", "r_pos") else (B, K)
+        if name not in OPTIONAL_OUTPUTS + EXPLORE_OUTPUTS:
+            raise ValueError(f"unknown output {name!r}; choose from {OPTIONAL_OUTPUTS + EXPLORE_OUTPUTS}")
+        shape = (B,) if name in ("nll", "entropy") else (B, K, T) if name in ("samples", "to_go", "r_pos") else (B, K)
         out[name] = torch.empty(shape, dtype=_OUT_DTYPES[name], device=dev)
     return out
 
@@ -310,10 +313,10 @@ def _check_outputs(out, key, dev):
     for name, t in out.items():
         if name in ("workspace",):
             continue
-        if name not in OPTIONAL_OUTPUTS + ("loss", "dlogits"):
+        if name not in OPTIONAL_OUTPUTS + EXPLORE_OUTPUTS + ("loss", "dlogits"):
             raise ValueError(f"unknown output {name!r}")
         want_dt = torch.float32 if name in ("loss", "dlogits") else _OUT_DTYPES[name]
-        n = 1 if name == "loss" else B * T * V if name == "dlogits" else B if name == "nll" else \
+        n = 1 if name == "loss" else B * T * V if name == "dlogits" else B if name in ("nll", "entropy") else \
             B * K * T if name in ("samples", "to_go", "r_pos") else B * K
         if not (isinstance(t, torch.Tensor) and t.device == dev and t.dtype == want_dt and t.is_contiguous()
                 and t.numel() == n):
@@ -351,30 +354,59 @@ def _prep_batch(logits, targets, input_lengths, target_lengths, uniforms, K):
     return batch, (B, T, V, int(K), Lmax), dev
 
 
-def _step_entry(reward, blank, space_id):
-    """(entry point name, extra arguments before the workspace): the word rewards go through
-    pgasr_pg_ctc_step_multi_ws with the separator id, every other mode through pgasr_pg_ctc_step_multi."""
+def check_explore(temperature, entropy_weight, pg_weight, want_entropy=False):
+    """ValueError unless the exploration controls are valid (DESIGN.md "exploration spec"): temperature finite in
+    [0.01, 100], entropy_weight finite and >= 0; the entropy bonus and the entropy output need the PG term."""
+    t, w = float(temperature), float(entropy_weight)
+    if not (math.isfinite(t) and 0.01 <= t <= 100.0):
+        raise ValueError(f"temperature must be finite and in [0.01, 100], got {temperature!r}")
+    if not (math.isfinite(w) and w >= 0.0):
+        raise ValueError(f"entropy_weight must be finite and >= 0, got {entropy_weight!r}")
+    if (w > 0.0 or want_entropy) and float(pg_weight) == 0.0:
+        raise ValueError("the entropy bonus and the entropy output need the PG term (pg_weight != 0)")
+
+
+def _step_entry(reward, blank, space_id, temperature=1.0, entropy_weight=0.0, want_entropy=False):
+    """(entry point name, extra arguments before the workspace): non-default exploration controls or an entropy
+    output go through pgasr_pg_ctc_step_multi_ex (its extra arguments follow the per-step entropy pointer array:
+    word_sep, temperature, w_ent); otherwise the word rewards go through pgasr_pg_ctc_step_multi_ws with the
+    separator id, every other mode through pgasr_pg_ctc_step_multi."""
     if reward not in REWARD_MODES:
         raise ValueError(f"unknown reward {reward!r}; choose from {tuple(REWARD_MODES)}")
+    if reward in WORD_REWARDS:
+        if space_id is None:
+            raise ValueError(f"reward={reward!r} needs space_id, the id of the word separator (the space character)")
+        if int(space_id) == int(blank):
+            raise ValueError("space_id must differ from blank")
+    if float(temperature) != 1.0 or float(entropy_weight) != 0.0 or want_entropy:
+        sep = int(space_id) if reward in WORD_REWARDS else -1
+        return "pgasr_pg_ctc_step_multi_ex", (sep, float(temperature), float(entropy_weight))
     if reward not in WORD_REWARDS:
         return "pgasr_pg_ctc_step_multi", ()
-    if space_id is None:
-        raise ValueError(f"reward={reward!r} needs space_id, the id of the word separator (the space character)")
-    if int(space_id) == int(blank):
-        raise ValueError("space_id must differ from blank")
     return "pgasr_pg_ctc_step_multi_ws", (int(space_id),)
+
+
+def _entropy_ptrs(outs):
+    """The host array of per-step entropy pointers of pgasr_pg_ctc_step_multi_ex (NULL where not wanted)."""
+    return (C.c_void_p * len(outs))(*[_ptr(o.get("entropy")) for o in outs])
 
 
 def pg_ctc_step(logits, targets, input_lengths=None, target_lengths=None, K=16, blank=0, reward="ed",
                 baseline="mean", baseline_value=0.0, pg_weight=1.0, ctc_weight=1.0, uniforms=None, seed=0,
-                workspace=None, want=("rewards", "nll"), out=None, space_id=None):
+                workspace=None, want=("rewards", "nll"), out=None, space_id=None, temperature=1.0,
+                entropy_weight=0.0):
     """The whole loss step (rows a1-a8 chained) in one C-ABI call.
     Returns a dict: loss (0-d), dlogits [B,T,V], plus the optional outputs named in `want` out of
     rewards, logp, hyp_len, dist, nll, samples (and, with reward='ed_to_go', to_go and r_pos [B,K,T]).
     `out`: a dict from StepWorkspace.outputs() to write into instead of allocating (no allocation per step).
     reward='wed' / 'wer' (word edit distance, -WED / n_words): space_id is the id of the word separator; dist then
-    holds word edit distances (hyp_len stays in ids)."""
-    entry, extra = _step_entry(reward, blank, space_id)
+    holds word edit distances (hyp_len stays in ids).
+    temperature / entropy_weight (DESIGN.md "exploration spec"): the PG term samples from and trains
+    softmax(logits / temperature) and the loss gains -entropy_weight * mean_b H_b; 'entropy' in `want` returns H_b [B]
+    (nats, summed over the utterance's frames).  The CTC term always uses the untempered logits."""
+    want_entropy = "entropy" in (out if out is not None else want)
+    check_explore(temperature, entropy_weight, pg_weight, want_entropy)
+    entry, extra = _step_entry(reward, blank, space_id, temperature, entropy_weight, want_entropy)
     batch, key, dev = _prep_batch(logits, targets, input_lengths, target_lengths, uniforms, K)
     B, T, V, K, Lmax = key
     if workspace is None or workspace.key != key or workspace.device != dev:
@@ -384,8 +416,9 @@ def pg_ctc_step(logits, targets, input_lengths=None, target_lengths=None, K=16, 
     else:
         _check_outputs(out, key, dev)
     io = _step_io(batch, out, seed)
+    ent = (_entropy_ptrs([out]),) if entry == "pgasr_pg_ctc_step_multi_ex" else ()
     _launch(logits, entry, C.byref(io), 1, 0, B, T, V, K, Lmax, int(blank), REWARD_MODES[reward],
-            BASELINE_MODES[baseline], float(baseline_value), float(pg_weight), float(ctc_weight), *extra,
+            BASELINE_MODES[baseline], float(baseline_value), float(pg_weight), float(ctc_weight), *ent, *extra,
             _ptr(workspace.buf), workspace.nbytes)
     res = dict(out)
     res["loss"] = out["loss"][0]
@@ -403,8 +436,10 @@ class StepQueue:
     """
 
     def __init__(self, batches, K=16, blank=0, reward="ed", baseline="mean", baseline_value=0.0, pg_weight=1.0,
-                 ctc_weight=1.0, want=("rewards", "nll"), workspace=None, space_id=None):
-        self._entry, self._extra = _step_entry(reward, blank, space_id)
+                 ctc_weight=1.0, want=("rewards", "nll"), workspace=None, space_id=None, temperature=1.0,
+                 entropy_weight=0.0):
+        check_explore(temperature, entropy_weight, pg_weight, "entropy" in want)
+        self._entry, self._extra = _step_entry(reward, blank, space_id, temperature, entropy_weight, "entropy" in want)
         if not batches:
             raise ValueError("StepQueue needs at least one batch")
         self.batches, self.outputs = [], []
@@ -430,6 +465,8 @@ class StepQueue:
         for i in range(2 * n):
             self._io[i] = _step_io(self.batches[i % n], self.outputs[i % n], seed=i)
         self._stride = C.sizeof(_native.StepIO)
+        # pgasr_pg_ctc_step_multi_ex: the entropy pointers, doubled like the records
+        self._ent = _entropy_ptrs(self.outputs * 2) if self._entry == "pgasr_pg_ctc_step_multi_ex" else None
 
     def run(self, first=0, n=None, seed=0):
         """Enqueue steps on batches first, first+1, ... (cyclically), n <= len(batches) of them; returns n."""
@@ -440,6 +477,7 @@ class StepQueue:
         first = int(first) % nb
         B, T, V, K, Lmax = self.key
         base = C.addressof(self._io) + first * self._stride
+        ent = () if self._ent is None else (C.addressof(self._ent) + first * C.sizeof(C.c_void_p),)
         _launch(self.workspace.buf, self._entry, base, n, (int(seed) - first) & (2**64 - 1), B, T, V, K,
-                Lmax, *self.params, *self._extra, _ptr(self.workspace.buf), self.workspace.nbytes)
+                Lmax, *self.params, *ent, *self._extra, _ptr(self.workspace.buf), self.workspace.nbytes)
         return n

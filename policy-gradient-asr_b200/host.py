@@ -40,9 +40,12 @@ def _host(t, dtype, name, numel=None, optional=False):
 
 class HostPipeline:
     def __init__(self, B, T, V, K, Lmax, depth=3, blank=0, reward="ed", baseline="mean", baseline_value=0.0,
-                 pg_weight=1.0, ctc_weight=1.0):
+                 pg_weight=1.0, ctc_weight=1.0, temperature=1.0, entropy_weight=0.0):
         if reward in WORD_REWARDS:
             raise ValueError(f"reward={reward!r} (word level) is not available on host buffers; use "
+                             "functional.pg_ctc_step or PolicyGradCTCLoss with device tensors")
+        if float(temperature) != 1.0 or float(entropy_weight) != 0.0:
+            raise ValueError("temperature and entropy_weight are not available on host buffers; use "
                              "functional.pg_ctc_step or PolicyGradCTCLoss with device tensors")
         self.shape = (int(B), int(T), int(V), int(K), int(Lmax))
         self.depth = int(depth)

@@ -48,10 +48,10 @@ class _PGCTCFn(torch.autograd.Function):
                             blank=module.blank, reward=module.reward, baseline=module.baseline,
                             baseline_value=module.baseline_value, pg_weight=module.pg_weight,
                             ctc_weight=module.ctc_weight, uniforms=uniforms, seed=module._next_seed(),
-                            space_id=module.space_id,
-                            workspace=module._workspace, want=("rewards", "nll", "logp", "dist", "hyp_len"))
+                            space_id=module.space_id, temperature=module.temperature,
+                            entropy_weight=module.entropy_weight, workspace=module._workspace, want=module._want)
         module._workspace = out["workspace"]
-        module.last = {k: out[k] for k in ("rewards", "nll", "logp", "dist", "hyp_len")}
+        module.last = {k: out[k] for k in module._want}
         ctx.save_for_backward(out["dlogits"])
         return out["loss"]
 
@@ -62,7 +62,8 @@ class _PGCTCFn(torch.autograd.Function):
 
 
 class PolicyGradCTCLoss(nn.Module):
-    """loss = pg_weight * L_pg + ctc_weight * mean_b nll_b   (DESIGN.md "policy gradient spec", "CTC spec")
+    """loss = pg_weight * L_pg + ctc_weight * mean_b nll_b - entropy_weight * mean_b H_b
+    (DESIGN.md "policy gradient spec", "CTC spec", "exploration spec")
 
     forward(logits[B,T,V] fp32 CUDA, targets[B,L] (pad 0), input_lengths[B]=None, target_lengths[B]=None,
             uniforms[B,K,T]=None) -> 0-d tensor attached to `logits`.
@@ -76,13 +77,18 @@ class PolicyGradCTCLoss(nn.Module):
     target_lengths=None: the lengths are taken from the padding -- the number of leading non-zero ids of each row
             (upstream pads transcripts with 0 = '<pad>', data.py:99, which is also the CTC blank and never a label)
     baseline: 'mean' (over the K samples of the utterance), 'loo', 'none', or 'value' (baseline_value)
+    temperature: the PG term samples from and trains softmax(logits / temperature) (finite, 0.01..100); the CTC term
+            keeps the untempered logits
+    entropy_weight: weight of the entropy bonus (finite, >= 0; > 0 needs pg_weight != 0); H_b is the entropy of the
+            tempered policy summed over the utterance's frames, in nats
     After a call, .last holds rewards [B,K], nll [B], logp [B,K], dist [B,K] (word edit distances for 'wed' / 'wer'),
-    hyp_len [B,K].
+    hyp_len [B,K], and entropy [B] (H_b) when temperature or entropy_weight is not the default.
     """
 
     def __init__(self, K=16, blank=0, reward="ed", baseline="mean", baseline_value=0.0, pg_weight=1.0,
-                 ctc_weight=1.0, seed=0, space_id=None):
+                 ctc_weight=1.0, seed=0, space_id=None, temperature=1.0, entropy_weight=0.0):
         super().__init__()
+        F.check_explore(temperature, entropy_weight, pg_weight)
         if reward not in F.REWARD_MODES or baseline not in F.BASELINE_MODES:
             raise ValueError("unknown reward or baseline mode")
         if reward in F.WORD_REWARDS:
@@ -93,6 +99,10 @@ class PolicyGradCTCLoss(nn.Module):
         self.space_id = None if space_id is None else int(space_id)
         self.K, self.blank, self.reward, self.baseline = int(K), int(blank), reward, baseline
         self.baseline_value, self.pg_weight, self.ctc_weight = float(baseline_value), float(pg_weight), float(ctc_weight)
+        self.temperature, self.entropy_weight = float(temperature), float(entropy_weight)
+        self._want = ("rewards", "nll", "logp", "dist", "hyp_len")
+        if (self.temperature != 1.0 or self.entropy_weight != 0.0) and self.pg_weight != 0.0:
+            self._want += ("entropy",)
         self.seed, self._calls = int(seed), 0
         self._workspace = None
         self.last = {}
