@@ -30,6 +30,9 @@
  *   in_len [B], tgt_len [B] int32               uniforms [B,K,T] fp32 in [0,1)
  *   samples / hyps [B,K,T] uint8 (V <= 256)     hyp_len / dist [B,K] int32
  *   logp / rewards / adv [B,K] fp32             nll [B] fp32
+ * Alignment: an array argument needs only its element's natural alignment (4 bytes for fp32 / int32, 2 for int16, 1
+ * for uint8), so a view at any element offset into a larger buffer is a valid argument; wider accesses are taken only
+ * where the pointer allows them.  Workspaces are the exception: 256-byte aligned.
  */
 #ifndef PGASR_H_
 #define PGASR_H_

@@ -225,7 +225,9 @@ __device__ void fused_ctc_role(const FusedArgs& a, int b, unsigned char* smem_ra
         {
             float* stage = reinterpret_cast<float*>(stage_base);
             const int chunk = stage_chunk;
-            const bool al16 = (((size_t)T * V * 4) & 15) == 0;
+            // (any float* is a valid logits pointer: the 16-byte copies need the base aligned too.  Every utterance's
+            // base differs by T*V*4 bytes, so the predicate is the same for all of them)
+            const bool al16 = ((reinterpret_cast<uintptr_t>(lg) | ((size_t)T * V * 4)) & 15) == 0;
             for (int c0 = 0; c0 < Tb; c0 += chunk) {
                 const int n = min(chunk, Tb - c0);
                 const float* src = lg + (size_t)c0 * V;
@@ -533,7 +535,7 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
         if (!kStream && a.bulk_tile) {
             if (threadIdx.x == 0) bulk_load_tile(ztile, lg, (unsigned)((size_t)T * V * 4), s_mbar);
         } else if (!kStream) {
-            if ((((size_t)T * V * 4) & 15) == 0) {
+            if (((reinterpret_cast<uintptr_t>(lg) | ((size_t)T * V * 4)) & 15) == 0) {
                 const int n16 = T * V / 4;
                 for (int i = threadIdx.x; i < n16; i += kThreads)
                     cp_async16(reinterpret_cast<char*>(ztile) + (size_t)i * 16, reinterpret_cast<const char*>(lg) + (size_t)i * 16);
@@ -1341,7 +1343,7 @@ __device__ void fused_pg_role(const FusedArgs& a, int b0, int nutt, unsigned cha
         }
         __syncthreads();
         PGASR_STAMP(dbg, 37);
-        if ((((size_t)T * V * 4) & 15) == 0) {
+        if (((reinterpret_cast<uintptr_t>(dlog_u) | ((size_t)T * V * 4)) & 15) == 0) {   // (dlogits: any float*)
             float4* d4 = reinterpret_cast<float4*>(dlog_u);
             const float4* t4 = reinterpret_cast<const float4*>(ztile);
             const int n4 = T * V / 4;

@@ -14,8 +14,7 @@ import torch
 
 from oracle import cport
 from tests import explore_ref
-from tests.synth import make_batch
-from tests.test_word_reward import make_word_batch
+from tests.synth import make_batch, make_word_batch
 
 RTOL = 1e-4
 REWARDS = ("ed", "cer", "ed_to_go", "wed", "wer")
