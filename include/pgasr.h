@@ -55,7 +55,7 @@ extern "C" {
 typedef enum {
     PGASR_OK = 0,
     PGASR_ERR_INVALID_ARG = -1,   /* NULL pointer, negative size, size over a documented limit */
-    PGASR_ERR_UNSUPPORTED = -2,   /* legal request this build has no kernel for (e.g. V > 64 sampler) */
+    PGASR_ERR_UNSUPPORTED = -2,   /* legal request this build has no kernel for (e.g. V > 256 sampler) */
     PGASR_ERR_NO_DEVICE = -3,     /* no CUDA device of compute capability 10.x */
     PGASR_ERR_WORKSPACE = -4,     /* workspace too small; ask pgasr_*_workspace_bytes */
     PGASR_ERR_CUDA = -5           /* a CUDA call failed; pgasr_last_cuda_error() has the code */
@@ -85,7 +85,8 @@ PGASR_API int         pgasr_device_check(void);             /* PGASR_OK iff the 
  * samples[b,k,t] ~ Categorical(softmax(logits[b,t,:])) for t < in_len[b] (0 beyond), from
  * uniforms[b,k,t] when given, else Philox4x32-10(seed; counter (t, b, k/4, 'PGAS'), lane k%4).
  * logp[b,k] = sum_t log_softmax(logits[b,t,:])[samples[b,k,t]].  probs (optional) receives the
- * softmax.  Bit-exact contract: DESIGN.md "sampler spec".  V <= 64, K <= 64.                   */
+ * softmax.  Bit-exact contract: DESIGN.md "sampler spec".  V <= 256, K <= 64: rows in registers for
+ * V <= 64, rows and CDF in shared memory above.                                                */
 PGASR_API int pgasr_softmax_sample(const float* logits, const int32_t* in_len, const float* uniforms,
                          uint64_t seed, int B, int T, int V, int K,
                          uint8_t* samples, float* logp, float* probs, void* stream);
@@ -135,7 +136,8 @@ PGASR_API int pgasr_pg_grad(const uint8_t* samples, const float* adv, const floa
  * probs: softmax of logits if the caller already has it (pgasr_softmax_sample), else NULL and the
  * kernel computes it into its workspace.  No valid alignment: nll = +inf, zero gradient.
  * With logits given, accumulate == 0 and V <= 64 this is the CTC role of the single-launch kernel below (walker and
- * gradient-worker warps, any T); otherwise the classic one-CTA-per-utterance kernel.
+ * gradient-worker warps, any T); otherwise the classic one-CTA-per-utterance kernel (V <= 256: 32 staged frames
+ * per batch up to V = 196, 16 above).
  * Lmax <= 511.  workspace: pgasr_ctc_workspace_bytes(B,T,V,Lmax) bytes, 256-byte aligned.       */
 PGASR_API size_t pgasr_ctc_workspace_bytes(int B, int T, int V, int Lmax);
 PGASR_API int pgasr_ctc_loss_grad(const float* logits, const float* probs, const int32_t* targets,
@@ -165,9 +167,10 @@ PGASR_API int pgasr_nll_sum_backward(const int64_t* target, const float* grad_ou
  * serialisation: back-to-back steps on one stream overlap the launch of step n+1 with the tail of step n (the CTAs of
  * n+1 wait on the grid dependency before they touch any input or output); for that a lane holds two control blocks that
  * consecutive launches use alternately -- the library remembers, per lane pointer, which one is next (host side).
- * V <= 64 (register-resident fast paths up to 32 classes), K <= 64.  One kernel launch for every shape whose sample
- * buffers fit an SM (2.5 K T <= ~200 KB); targets / in_len / tgt_len and the small outputs may live in pinned host
- * memory mapped into the device (they are read once per CTA / written once).                       */
+ * V <= 256: one launch for V <= 64, a chain of stand-alone kernels above (register-resident fast paths up to 32
+ * classes; reward PGASR_REWARD_ED_TO_GO needs the single launch and is UNSUPPORTED above 64), K <= 64.  One kernel
+ * launch for every shape with V <= 64 whose sample buffers fit an SM (2.5 K T <= ~200 KB); targets / in_len /
+ * tgt_len and the small outputs may live in pinned host memory mapped into the device (they are read once per CTA / written once).                       */
 PGASR_API size_t pgasr_pg_ctc_step_workspace_bytes(int B, int T, int V, int K, int Lmax);
 /* (init also forgets which control block the workspace pointer used last, so a freed and recycled pointer is safe) */
 PGASR_API int pgasr_pg_ctc_step_workspace_init(void* workspace, size_t workspace_bytes, void* stream);
@@ -239,7 +242,9 @@ PGASR_API int pgasr_pg_ctc_step_multi_ex(const pgasr_step_io* steps, int n_steps
  * probs [N,T,V] fp64 post-softmax (upstream takes the post-softmax array and works in Python floats), frames
  * t >= in_len[n] ignored (in_len NULL: T).  labels [N,T] int32 receives the best prefix of each utterance (zero
  * filled beyond label_len[n]), nll[n] = -log(p_blank + p_non_blank) of that prefix, as upstream returns.
- * One CTA per utterance; V <= 64, beam <= 128.  workspace: pgasr_ctc_beam_search_workspace_bytes(N,T,V,beam).  */
+ * One CTA per utterance; V <= 256, beam <= 128, and the candidate table (beam (V + 1) doubles) in shared memory:
+ * beam <= 104 at V = 256.  workspace: pgasr_ctc_beam_search_workspace_bytes(N,T,V,beam), 0 for a shape the kernel
+ * does not take (the call then returns PGASR_ERR_UNSUPPORTED).  */
 PGASR_API size_t pgasr_ctc_beam_search_workspace_bytes(int N, int T, int V, int beam);
 PGASR_API int pgasr_ctc_beam_search(const double* probs, const int32_t* in_len, int N, int T, int V, int beam,
                           int blank, int32_t* labels, int32_t* label_len, double* nll,

@@ -46,7 +46,9 @@ def collapse_fn(preds):
 class CTCDecoder:
     """Prefix beam search with the upstream constructor and decode() signature
     (CTCdecoder.py:23-25, 41-116): decode(probs[T,V] post-softmax, beam_size=100, blank=0)
-    -> (labels tuple, negative log-likelihood), computed by the batched GPU kernel (csrc/beam.cu)."""
+    -> (labels tuple, negative log-likelihood), computed by the batched GPU kernel (csrc/beam.cu).
+    Alphabets of up to 256 classes, beams of up to 128 (up to 104 at 256 classes: the candidate table lives in
+    shared memory); larger requests raise PgasrError (status -2)."""
 
     def __init__(self, alphabet):
         self.alphabet = alphabet

@@ -22,7 +22,9 @@ namespace pgasr {
 
 constexpr int kBeamThreads = 128;
 constexpr int kBeamMax = 128;
-constexpr int kBeamMaxV = 64;
+constexpr int kBeamMaxV = 64;            // classes of the one-word symbol masks (ctc_beam_kernel)
+constexpr int kBeamWideWords = kMaxWideV / 64;   // mask words per slot of ctc_beam_wide_kernel (kBeamMaxV < V <= 256)
+constexpr size_t kBeamMaxSmem = 226 * 1024;  // dynamic shared memory a CTA may take (227 KB less the static part)
 
 __device__ __forceinline__ double lse2(double a, double b) {
     if (a == -INFINITY) return b;
@@ -34,14 +36,15 @@ __device__ __forceinline__ double lse2(double a, double b) {
 struct BeamSet {            // one generation of the beam, in shared memory
     double* pb; double* pnb;
     int* node; int* pnode; int* last; int* par;
-    unsigned long long* mask;
+    unsigned long long* mask;   // NW words per slot: bit s of slot i = (s >> 6, s & 63)
 };
 
+template <int NW>
 __device__ __forceinline__ BeamSet beam_carve(unsigned char*& p, int beam) {
     BeamSet b;
     b.pb = reinterpret_cast<double*>(p);                p += sizeof(double) * beam;
     b.pnb = reinterpret_cast<double*>(p);               p += sizeof(double) * beam;
-    b.mask = reinterpret_cast<unsigned long long*>(p);  p += sizeof(unsigned long long) * beam;
+    b.mask = reinterpret_cast<unsigned long long*>(p);  p += sizeof(unsigned long long) * NW * beam;
     b.node = reinterpret_cast<int*>(p);                 p += sizeof(int) * beam;
     b.pnode = reinterpret_cast<int*>(p);                p += sizeof(int) * beam;
     b.last = reinterpret_cast<int*>(p);                 p += sizeof(int) * beam;
@@ -49,12 +52,22 @@ __device__ __forceinline__ BeamSet beam_carve(unsigned char*& p, int beam) {
     return b;
 }
 
+// at V = 256 (4 mask words) this is 2188 beam + 2112 bytes: beams up to 104 fit kBeamMaxSmem
 static size_t beam_smem_bytes(int V, int beam) {
-    const size_t set = (size_t)beam * (3 * 8 + 4 * 4);
+    const int nw = V > kBeamMaxV ? kBeamWideWords : 1;
+    const size_t set = (size_t)beam * (2 * 8 + 8 * nw + 4 * 4);
     return 2 * set + sizeof(double) * (size_t)V + sizeof(double) * (size_t)beam * (V + 1) + sizeof(int) * (size_t)beam + 64;
 }
 
+// is s on slot i's children mask
+template <int NW>
+__device__ __forceinline__ bool beam_has_child(const BeamSet& b, int i, int s) {
+    if constexpr (NW == 1) return (b.mask[i] >> s) & 1ull;
+    else return (b.mask[i * NW + (s >> 6)] >> (s & 63)) & 1ull;
+}
+
 // (n_p_b, n_p_nb) of candidate c; see the header comment
+template <int NW>
 __device__ __forceinline__ void beam_candidate(const BeamSet& b, int nb, int beam, int V, int blank, const double* lp,
                                                int c, double& npb, double& npnb) {
     npb = npnb = -INFINITY;
@@ -75,7 +88,7 @@ __device__ __forceinline__ void beam_candidate(const BeamSet& b, int nb, int bea
         }
     } else {
         const int e = c - beam, s = e / beam, i = e - s * beam;
-        if (i >= nb || s == blank || s >= V || ((b.mask[i] >> s) & 1ull)) return;
+        if (i >= nb || s == blank || s >= V || beam_has_child<NW>(b, i, s)) return;
         const double y = lp[s];
         npnb = s != b.last[i] ? lse2(b.pb[i] + y, b.pnb[i] + y) : b.pb[i] + y;
     }
@@ -104,7 +117,9 @@ __device__ int beam_child(int parent, int s, unsigned long long* hkeys, int* hva
     }
 }
 
-__global__ void __launch_bounds__(kBeamThreads) ctc_beam_kernel(
+// one utterance; NW 64-bit words per children mask (the two kernels below)
+template <int NW>
+__device__ __forceinline__ void beam_utterance(
     const double* __restrict__ probs, const int32_t* __restrict__ in_len, int T, int V, int beam, int blank,
     int32_t* __restrict__ labels, int32_t* __restrict__ label_len, double* __restrict__ nll,
     int* node_parent_all, int* node_char_all, unsigned long long* hkeys_all, int* hvals_all, int maxn, int H) {
@@ -114,7 +129,7 @@ __global__ void __launch_bounds__(kBeamThreads) ctc_beam_kernel(
     __shared__ int s_widx[kBeamThreads / 32];
     const int u = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     unsigned char* p = smem;
-    BeamSet cur = beam_carve(p, beam), nxt = beam_carve(p, beam);
+    BeamSet cur = beam_carve<NW>(p, beam), nxt = beam_carve<NW>(p, beam);
     double* lp = reinterpret_cast<double*>(p);          p += sizeof(double) * V;
     double* score = reinterpret_cast<double*>(p);       p += sizeof(double) * (size_t)beam * (V + 1);
     int* sel = reinterpret_cast<int*>(p);
@@ -128,7 +143,8 @@ __global__ void __launch_bounds__(kBeamThreads) ctc_beam_kernel(
 
     if (tid == 0) {
         cur.pb[0] = 0.0; cur.pnb[0] = -INFINITY; cur.node[0] = 0; cur.pnode[0] = -1; cur.last[0] = -1; cur.par[0] = -1;
-        cur.mask[0] = 0ull;
+#pragma unroll
+        for (int w = 0; w < NW; ++w) cur.mask[w] = 0ull;
         node_parent[0] = -1; node_char[0] = -1;
         s_count = 1;
     }
@@ -144,7 +160,7 @@ __global__ void __launch_bounds__(kBeamThreads) ctc_beam_kernel(
         int best_c = 0x7fffffff;
         for (int c = tid; c < C; c += kBeamThreads) {
             double a, b2;
-            beam_candidate(cur, nb, beam, V, blank, lp, c, a, b2);
+            beam_candidate<NW>(cur, nb, beam, V, blank, lp, c, a, b2);
             const double sc = lse2(a, b2);
             score[c] = sc;
             if (sc > best) { best = sc; best_c = c; }
@@ -190,10 +206,11 @@ __global__ void __launch_bounds__(kBeamThreads) ctc_beam_kernel(
         for (int a = tid; a < m; a += kBeamThreads) {
             const int c = sel[a];
             double npb, npnb;
-            beam_candidate(cur, nb, beam, V, blank, lp, c, npb, npnb);
+            beam_candidate<NW>(cur, nb, beam, V, blank, lp, c, npb, npnb);
             nxt.pb[a] = npb;
             nxt.pnb[a] = npnb;
-            nxt.mask[a] = 0ull;
+#pragma unroll
+            for (int w = 0; w < NW; ++w) nxt.mask[a * NW + w] = 0ull;
             if (c < beam) {
                 nxt.node[a] = cur.node[c]; nxt.pnode[a] = cur.pnode[c]; nxt.last[a] = cur.last[c];
             } else {
@@ -211,7 +228,11 @@ __global__ void __launch_bounds__(kBeamThreads) ctc_beam_kernel(
                 for (int b2 = 0; b2 < m; ++b2)
                     if (nxt.node[b2] == pn) { par = b2; break; }
             nxt.par[a] = par;
-            if (par >= 0) atomicOr(nxt.mask + par, 1ull << nxt.last[a]);
+            if (par >= 0) {
+                const int s = nxt.last[a];
+                if constexpr (NW == 1) atomicOr(nxt.mask + par, 1ull << s);
+                else atomicOr(nxt.mask + par * NW + (s >> 6), 1ull << (s & 63));
+            }
         }
         __syncthreads();
         BeamSet tmp = cur; cur = nxt; nxt = tmp;
@@ -228,6 +249,23 @@ __global__ void __launch_bounds__(kBeamThreads) ctc_beam_kernel(
         for (int x = cur.node[0]; x > 0; x = node_parent[x]) labels[(size_t)u * T + --k] = node_char[x];
         for (int k2 = n; k2 < T; ++k2) labels[(size_t)u * T + k2] = 0;
     }
+}
+
+#define PGASR_BEAM_KERNEL(name, nw)                                                                                   \
+    __global__ void __launch_bounds__(kBeamThreads) name(                                                             \
+        const double* __restrict__ probs, const int32_t* __restrict__ in_len, int T, int V, int beam, int blank,      \
+        int32_t* __restrict__ labels, int32_t* __restrict__ label_len, double* __restrict__ nll,                      \
+        int* node_parent_all, int* node_char_all, unsigned long long* hkeys_all, int* hvals_all, int maxn, int H) {   \
+        beam_utterance<nw>(probs, in_len, T, V, beam, blank, labels, label_len, nll, node_parent_all, node_char_all,  \
+                           hkeys_all, hvals_all, maxn, H);                                                            \
+    }
+PGASR_BEAM_KERNEL(ctc_beam_kernel, 1)                   // V <= 64
+PGASR_BEAM_KERNEL(ctc_beam_wide_kernel, kBeamWideWords) // 64 < V <= 256
+#undef PGASR_BEAM_KERNEL
+
+// a shape the kernels take: V <= 256, beam <= 128, and the candidate table beam (V + 1) fits shared memory
+static bool beam_supported(int V, int beam) {
+    return V <= kMaxWideV && beam <= kBeamMax && beam_smem_bytes(V, beam) <= kBeamMaxSmem;
 }
 
 struct BeamWs { size_t parent, chr, keys, vals, total; int maxn, H; };
@@ -251,7 +289,7 @@ static BeamWs beam_ws(int N, int T, int beam) {
 
 extern "C" size_t pgasr_ctc_beam_search_workspace_bytes(int N, int T, int V, int beam) {
     using namespace pgasr;
-    if (N <= 0 || T <= 0 || V <= 0 || V > kBeamMaxV || beam <= 0 || beam > kBeamMax) return 0;
+    if (N <= 0 || T <= 0 || V <= 0 || beam <= 0 || !beam_supported(V, beam)) return 0;
     return beam_ws(N, T, beam).total;
 }
 
@@ -262,7 +300,7 @@ extern "C" int pgasr_ctc_beam_search(const double* probs, const int32_t* in_len,
     if (!probs || !labels || !label_len || !nll || !workspace || N <= 0 || T <= 0 || V <= 0 || beam <= 0 || blank < 0 ||
         blank >= V)
         return PGASR_ERR_INVALID_ARG;
-    if (V > kBeamMaxV || beam > kBeamMax) return PGASR_ERR_UNSUPPORTED;
+    if (!beam_supported(V, beam)) return PGASR_ERR_UNSUPPORTED;
     const BeamWs w = beam_ws(N, T, beam);
     if (workspace_bytes < w.total) return PGASR_ERR_WORKSPACE;
     cudaStream_t st = as_stream(stream);
@@ -273,9 +311,10 @@ extern "C" int pgasr_ctc_beam_search(const double* probs, const int32_t* in_len,
     int* node_char = reinterpret_cast<int*>(p);
     PGASR_CUDA_TRY(cudaMemsetAsync(hkeys, 0, w.keys, st));
     const size_t smem = beam_smem_bytes(V, beam);
-    PGASR_CUDA_TRY(cudaFuncSetAttribute(ctc_beam_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ctc_beam_kernel<<<N, kBeamThreads, smem, st>>>(probs, in_len, T, V, beam, blank, labels, label_len, nll, node_parent,
-                                                   node_char, hkeys, hvals, w.maxn, w.H);
+    const auto kern = V > kBeamMaxV ? ctc_beam_wide_kernel : ctc_beam_kernel;
+    PGASR_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<N, kBeamThreads, smem, st>>>(probs, in_len, T, V, beam, blank, labels, label_len, nll, node_parent, node_char,
+                                        hkeys, hvals, w.maxn, w.H);
     PGASR_LAUNCH_CHECK();
     return PGASR_OK;
 }

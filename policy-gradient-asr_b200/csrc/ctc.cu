@@ -26,13 +26,15 @@ namespace pgasr {
 
 constexpr int kCtcThreads = 128;  // warp 0: alpha, warp 1: beta, all four: softmax rows
 
-template <int SPL, bool kAccum>
-__global__ void __launch_bounds__(kCtcThreads)
-ctc_kernel(const float* __restrict__ logits, const float* __restrict__ probs_in,
-           double* __restrict__ probs_ws, const int32_t* __restrict__ targets,
-           const int32_t* __restrict__ in_len, const int32_t* __restrict__ tgt_len, int T, int V,
-           int Lmax, int blank, float grad_scale, float* __restrict__ nll,
-           float* __restrict__ dlogits, double* __restrict__ lattice, int* __restrict__ lat_exp) {
+// One utterance; kChunk frames per staged batch of each walking warp (kCtcChunk, or kCtcChunkWide for rows too wide
+// for it).  The two kernels below are this body with either depth.
+template <int SPL, bool kAccum, int kChunk>
+__device__ __forceinline__ void
+ctc_utterance(const float* __restrict__ logits, const float* __restrict__ probs_in,
+              double* __restrict__ probs_ws, const int32_t* __restrict__ targets,
+              const int32_t* __restrict__ in_len, const int32_t* __restrict__ tgt_len, int T, int V,
+              int Lmax, int blank, float grad_scale, float* __restrict__ nll,
+              float* __restrict__ dlogits, double* __restrict__ lattice, int* __restrict__ lat_exp) {
     extern __shared__ double smem_d[];
     const int b = blockIdx.x;
     const int warp = threadIdx.x >> 5;
@@ -58,18 +60,39 @@ ctc_kernel(const float* __restrict__ logits, const float* __restrict__ probs_in,
         mid();
         return;
     }
-    double* stage = smem_d + (size_t)warp * (2 * kCtcChunk * RS);
-    int* racc = reinterpret_cast<int*>(smem_d + (size_t)2 * (2 * kCtcChunk * RS)) + warp * (V + 2);
+    double* stage = smem_d + (size_t)warp * (2 * kChunk * RS);
+    int* racc = reinterpret_cast<int*>(smem_d + (size_t)2 * (2 * kChunk * RS)) + warp * (V + 2);
     double* lat_u = lattice + (size_t)b * T * (SPL * 32);
     int* exp_u = lat_exp + (size_t)b * T;
     const int32_t* lab_u = targets + (size_t)b * Lmax;
     if (warp == 0)
-        ctc_direction<SPL, true, kAccum, false>(pw, lab_u, Tb, L, V, RS, blank, grad_scale, nll + b, dlog_u, lat_u,
-                                                exp_u, stage, racc, mid);
+        ctc_direction<SPL, true, kAccum, false, kChunk>(pw, lab_u, Tb, L, V, RS, blank, grad_scale, nll + b, dlog_u,
+                                                        lat_u, exp_u, stage, racc, mid);
     else
-        ctc_direction<SPL, false, kAccum, false>(pw, lab_u, Tb, L, V, RS, blank, grad_scale, nll + b, dlog_u, lat_u,
-                                                 exp_u, stage, racc, mid);
+        ctc_direction<SPL, false, kAccum, false, kChunk>(pw, lab_u, Tb, L, V, RS, blank, grad_scale, nll + b, dlog_u,
+                                                         lat_u, exp_u, stage, racc, mid);
 }
+
+#define PGASR_CTC_KERNEL(name, chunk)                                                                                 \
+    template <int SPL, bool kAccum>                                                                                   \
+    __global__ void __launch_bounds__(kCtcThreads)                                                                    \
+    name(const float* __restrict__ logits, const float* __restrict__ probs_in, double* __restrict__ probs_ws,         \
+         const int32_t* __restrict__ targets, const int32_t* __restrict__ in_len, const int32_t* __restrict__ tgt_len, \
+         int T, int V, int Lmax, int blank, float grad_scale, float* __restrict__ nll, float* __restrict__ dlogits,   \
+         double* __restrict__ lattice, int* __restrict__ lat_exp) {                                                   \
+        ctc_utterance<SPL, kAccum, chunk>(logits, probs_in, probs_ws, targets, in_len, tgt_len, T, V, Lmax, blank,    \
+                                          grad_scale, nll, dlogits, lattice, lat_exp);                                \
+    }
+PGASR_CTC_KERNEL(ctc_kernel, kCtcChunk)           // V <= 196: 32 frames per batch
+PGASR_CTC_KERNEL(ctc_wide_kernel, kCtcChunkWide)  // 196 < V <= 256: 16 frames per batch
+#undef PGASR_CTC_KERNEL
+
+// dynamic shared memory of the classic kernel: two warps x two staged batches of kChunk rows, and the two warps'
+// label-column accumulators
+static size_t ctc_smem_bytes(int V, int chunk) {
+    return (size_t)2 * (2 * chunk * ctc_row_stride(V)) * sizeof(double) + (size_t)2 * (V + 2) * sizeof(int);
+}
+constexpr size_t kCtcMaxSmem = 200 * 1024;
 
 struct CtcWs { size_t lat, probs, exps, total; };
 static CtcWs ctc_ws(int B, int T, int V, int spl) {
@@ -88,20 +111,17 @@ static int launch_ctc(const float* logits, const float* probs, const int32_t* ta
     double* lattice = reinterpret_cast<double*>(base);
     double* probs_ws = reinterpret_cast<double*>(base + w.lat);
     int* lat_exp = reinterpret_cast<int*>(base + w.lat + w.probs);
-    const int RS = ctc_row_stride(V);
-    const size_t smem = (size_t)2 * (2 * kCtcChunk * RS) * sizeof(double) + (size_t)2 * (V + 2) * sizeof(int);
-    if (smem > 200 * 1024) return PGASR_ERR_UNSUPPORTED;
-    if (accumulate) {
-        if (smem > 48 * 1024)
-            PGASR_CUDA_TRY(cudaFuncSetAttribute(ctc_kernel<SPL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        ctc_kernel<SPL, true><<<B, kCtcThreads, smem, st>>>(logits, probs, probs_ws, targets, in_len, tgt_len, T, V,
-                                                            Lmax, blank, grad_scale, nll, dlogits, lattice, lat_exp);
-    } else {
-        if (smem > 48 * 1024)
-            PGASR_CUDA_TRY(cudaFuncSetAttribute(ctc_kernel<SPL, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        ctc_kernel<SPL, false><<<B, kCtcThreads, smem, st>>>(logits, probs, probs_ws, targets, in_len, tgt_len, T, V,
-                                                             Lmax, blank, grad_scale, nll, dlogits, lattice, lat_exp);
-    }
+    // 32 staged frames per batch while they fit (every V <= 196), else 16
+    const bool wide = ctc_smem_bytes(V, kCtcChunk) > kCtcMaxSmem;
+    const size_t smem = ctc_smem_bytes(V, wide ? kCtcChunkWide : kCtcChunk);
+    if (smem > kCtcMaxSmem) return PGASR_ERR_UNSUPPORTED;
+    using Kern = void (*)(const float*, const float*, double*, const int32_t*, const int32_t*, const int32_t*, int, int,
+                          int, int, float, float*, float*, double*, int*);
+    const Kern k = wide ? (accumulate ? ctc_wide_kernel<SPL, true> : ctc_wide_kernel<SPL, false>)
+                        : (accumulate ? ctc_kernel<SPL, true> : ctc_kernel<SPL, false>);
+    if (smem > 48 * 1024) PGASR_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<B, kCtcThreads, smem, st>>>(logits, probs, probs_ws, targets, in_len, tgt_len, T, V, Lmax, blank, grad_scale,
+                                    nll, dlogits, lattice, lat_exp);
     PGASR_LAUNCH_CHECK();
     return PGASR_OK;
 }

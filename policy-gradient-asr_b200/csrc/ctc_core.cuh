@@ -6,6 +6,7 @@
 namespace pgasr {
 
 constexpr int kCtcChunk = 32;     // frames staged per cp.async batch (staged mode); must be even
+constexpr int kCtcChunkWide = 16; // the same for rows too wide for kCtcChunk frames (ctc.cu: V > 196)
 
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
     unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
@@ -218,7 +219,7 @@ __device__ __forceinline__ void ctc_step(CtcLane<SPL>& st, GradNorm& gn, int ste
 
 // Steps [step_lo, step_hi) of one direction.  kTile: `probs` is a shared-memory tile [Tb][RS] of the whole
 // utterance; else it is the global fp64 workspace and rows are staged through `stage` with cp.async.
-template <int SPL, bool kAlpha, bool kGrad, bool kAccum, bool kTile>
+template <int SPL, bool kAlpha, bool kGrad, bool kAccum, bool kTile, int kChunk = kCtcChunk>
 __device__ __forceinline__ void ctc_frames(CtcLane<SPL>& st, GradNorm& gn, int step_lo, int step_hi, int Tb, int S,
                                            int V, int RS, int blank, const double* probs,
                                            double* __restrict__ lat_u, int* __restrict__ exp_u, float grad_scale,
@@ -254,18 +255,18 @@ __device__ __forceinline__ void ctc_frames(CtcLane<SPL>& st, GradNorm& gn, int s
     }
 
     auto issue_chunk = [&](int lo, int buf) {             // steps [lo, hi) -> contiguous frames
-        const int hi = min(lo + kCtcChunk, step_hi);
+        const int hi = min(lo + kChunk, step_hi);
         const int f0 = kAlpha ? lo : Tb - hi;
         const char* src = reinterpret_cast<const char*>(probs + (size_t)f0 * RS);
-        char* dst = reinterpret_cast<char*>(stage + (size_t)buf * kCtcChunk * RS);
+        char* dst = reinterpret_cast<char*>(stage + (size_t)buf * kChunk * RS);
         const int n16 = (hi - lo) * RS / 2;
         for (int i = lane; i < n16; i += 32) cp_async16(dst + (size_t)i * 16, src + (size_t)i * 16);
         cp_async_commit();
     };
     int buf = 0;
     issue_chunk(step_lo, 0);
-    for (int lo = step_lo; lo < step_hi; lo += kCtcChunk, buf ^= 1) {
-        const int hi = min(lo + kCtcChunk, step_hi);
+    for (int lo = step_lo; lo < step_hi; lo += kChunk, buf ^= 1) {
+        const int hi = min(lo + kChunk, step_hi);
         if (hi < step_hi) {
             issue_chunk(hi, buf ^ 1);
             cp_async_wait<1>();
@@ -273,7 +274,7 @@ __device__ __forceinline__ void ctc_frames(CtcLane<SPL>& st, GradNorm& gn, int s
             cp_async_wait<0>();
         }
         __syncwarp();
-        const double* chunk = stage + (size_t)buf * kCtcChunk * RS;
+        const double* chunk = stage + (size_t)buf * kChunk * RS;
         int step = lo;
         for (; step + 1 < hi; step += 2) {                // chunks hold an even number of frames except the last
             const int t = kAlpha ? step : Tb - 1 - step;
@@ -298,7 +299,7 @@ __device__ __forceinline__ void ctc_frames(CtcLane<SPL>& st, GradNorm& gn, int s
 // One whole direction: first half (store), mid-point barrier, second half (gradient rows), and for alpha the
 // negative log-likelihood.  `mid_barrier()` must synchronise the alpha and the beta warp (and make their global
 // stores visible to each other).
-template <int SPL, bool kAlpha, bool kAccum, bool kTile, typename Barrier>
+template <int SPL, bool kAlpha, bool kAccum, bool kTile, int kChunk, typename Barrier>
 __device__ __forceinline__ void ctc_direction(const double* probs, const int32_t* __restrict__ lab_u, int Tb, int L,
                                               int V, int RS, int blank, float grad_scale,
                                               float* __restrict__ nll_out, float* __restrict__ dlog_u,
@@ -315,10 +316,10 @@ __device__ __forceinline__ void ctc_direction(const double* probs, const int32_t
     gn.have = false; gn.dead = false; gn.invZ0 = 0.0; gn.E0 = 0;
     // steps 0..Tb-1 visit frames 0..Tb-1 (alpha) or Tb-1..0 (beta)
     const int n_first = kAlpha ? tm : Tb - tm;
-    ctc_frames<SPL, kAlpha, false, kAccum, kTile>(st, gn, 0, n_first, Tb, S, V, RS, blank, probs, lat_u, exp_u,
+    ctc_frames<SPL, kAlpha, false, kAccum, kTile, kChunk>(st, gn, 0, n_first, Tb, S, V, RS, blank, probs, lat_u, exp_u,
                                                   grad_scale, dlog_u, stage, racc);
     mid_barrier();
-    ctc_frames<SPL, kAlpha, true, kAccum, kTile>(st, gn, n_first, Tb, Tb, S, V, RS, blank, probs, lat_u, exp_u,
+    ctc_frames<SPL, kAlpha, true, kAccum, kTile, kChunk>(st, gn, n_first, Tb, Tb, S, V, RS, blank, probs, lat_u, exp_u,
                                                  grad_scale, dlog_u, stage, racc);
     if (kAlpha) {
         double fin = 0.0;

@@ -39,7 +39,9 @@ static __device__ long long g_dbg[64];   // one copy per translation unit; fused
 #define PGASR_ACCUM(cond, slot, v) do { } while (0)
 #endif
 
-constexpr int kMaxV = 64;         // classes the sampler, the fused step and the host pipeline take (fast paths: V <= 32)
+constexpr int kMaxV = 64;         // classes the fused step and the host pipeline take (fast paths: V <= 32)
+constexpr int kMaxWideV = 256;    // classes the sampler, the step (chain of stand-alone kernels above kMaxV) and the
+                                  // beam search take: the uint8 sample format's limit
 constexpr int kWarp = 32;
 constexpr unsigned kFull = 0xffffffffu;
 

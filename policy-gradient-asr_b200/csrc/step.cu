@@ -167,7 +167,7 @@ static int step_check(const StepParams& q, const void* workspace, size_t workspa
     if (q.reward_mode < 0 || (q.reward_mode > PGASR_REWARD_MAX && !(words && word_mode(q.reward_mode))) ||
         q.baseline_mode < 0 || q.baseline_mode > 3)
         return PGASR_ERR_INVALID_ARG;
-    if (q.K > 64 || q.V > kMaxV) return PGASR_ERR_UNSUPPORTED;
+    if (q.K > 64 || q.V > kMaxWideV) return PGASR_ERR_UNSUPPORTED;
     const size_t need = pgasr_pg_ctc_step_workspace_bytes(q.B, q.T, q.V, q.K, q.Lmax);
     if (need == 0) return PGASR_ERR_UNSUPPORTED;
     if (workspace_bytes < need) return PGASR_ERR_WORKSPACE;

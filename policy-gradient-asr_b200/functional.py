@@ -67,7 +67,8 @@ def as_targets(targets, device):
 
 
 def softmax_sample(logits, input_lengths=None, K=16, uniforms=None, seed=0, return_probs=False):
-    """Row a6.  logits [B,T,V] fp32 -> samples [B,K,T] uint8, logp [B,K] fp32 (and probs [B,T,V])."""
+    """Row a6.  logits [B,T,V] fp32 -> samples [B,K,T] uint8, logp [B,K] fp32 (and probs [B,T,V]).
+    V <= 256 classes, K <= 64 draws."""
     logits = _need(logits, torch.float32, "logits", 3)
     B, T, V = logits.shape
     if uniforms is not None:
@@ -264,7 +265,8 @@ def ctc_beam_search(probs, input_lengths=None, beam_size=100, blank=0):
     in_len = _opt_i32(input_lengths, "input_lengths", N, probs.device)
     nbytes = _native.lib().pgasr_ctc_beam_search_workspace_bytes(N, T, V, int(beam_size))
     if nbytes == 0:
-        raise _native.PgasrError("pgasr_ctc_beam_search_workspace_bytes", -2, "unsupported size (V <= 64, beam <= 128)")
+        raise _native.PgasrError("pgasr_ctc_beam_search_workspace_bytes", -2,
+                                 "unsupported size (V <= 256, beam <= 128; beam <= 104 at V = 256)")
     ws = torch.empty((nbytes,), dtype=torch.uint8, device=probs.device)
     labels = torch.empty((N, T), dtype=torch.int32, device=probs.device)
     label_len = torch.empty((N,), dtype=torch.int32, device=probs.device)

@@ -67,6 +67,8 @@ class PolicyGradCTCLoss(nn.Module):
 
     forward(logits[B,T,V] fp32 CUDA, targets[B,L] (pad 0), input_lengths[B]=None, target_lengths[B]=None,
             uniforms[B,K,T]=None) -> 0-d tensor attached to `logits`.
+    V: up to 256 classes.  V <= 64 runs the single-launch kernel; wider alphabets run a chain of stand-alone kernels
+            (same results, more launches; 'ed_to_go' needs the single-launch kernel and is refused above 64 classes)
     reward: 'ed' (-edit distance), 'cer' (-edit distance / len(transcript), as metrics.evaluate's CER) or
             'ed_to_go' (upstream policy_grad.reward's per-position rewards, credited per frame as reward-to-go;
             the baseline is then taken per frame over the K samples),
